@@ -2,6 +2,7 @@
 """bench.py -- nucleotides/s through HyenaOperator fwd+bwd at L=1,048,576, d_model=256 (BASELINE.json).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's sm_100a path
+    python bench.py --steps K --dump-outputs DIR                   # ... and write the last timed step's outputs
     python bench.py --impl reference [--steps K] [--warmup W]      # the reference's CPU torch.fft path
 
 A "step" is one forward + backward of the operator over one batch of synthetic single-nucleotide
@@ -62,7 +63,33 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--e2e-chunks", type=int, default=4, help="sequence chunks of the HostStep copy pipeline")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write y, du and the parameter grads of the last timed step as DIR/<name>.npy (rank 0)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+# ----------------------------------------------------------------------------------------- output dump
+DUMP_BYTES = 60 * 10 ** 6        # payload of --dump-outputs in all (npy headers stay well inside 64 MB)
+
+
+def dump_outputs(outdir, outputs, seed=0):
+    """outputs: {name: tensor}.  Writes DIR/<name>.npy (float32, float64 kept).  Each output gets an equal share of
+    DUMP_BYTES: one that fits is written whole, a larger one as a 1-D array of its entries at a fixed seeded sample of
+    its flat indices (sorted; the same indices for every output of one size), so that two runs with the same arguments
+    are comparable array for array."""
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    for name, t in outputs.items():
+        t = t.detach()
+        share = DUMP_BYTES // len(outputs) // (8 if t.dtype == torch.float64 else 4)      # elements
+        if t.numel() > share:
+            idx = np.unique(np.random.default_rng(seed).integers(0, t.numel(), share))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        a = t.cpu().numpy()
+        np.save(os.path.join(outdir, name + ".npy"), a if a.dtype == np.float64 else a.astype(np.float32))
 
 
 # ----------------------------------------------------------------------------------------- clocks
@@ -284,41 +311,17 @@ def reference_arm(args):
 
 # ----------------------------------------------------------------------------------------- reference GPU path
 def gpu_reference_run(op, u, dy, steps=3, warmup=1):
-    """The reference's own GPU path (plain torch ops: F.linear, F.conv1d, torch.fft -> cuFFT; hyena.py:388-444) on the
-    same device, same weights, same inputs, fp32 with TF32 off: the >=10x denominator of north_star.  Imports the
-    UNMODIFIED reference module when /root/reference exists (build container), else runs the oracle restatement of it
-    on cuda (the GPU box has no /root/reference)."""
+    """The reference's own GPU path (plain torch ops: F.linear, F.conv1d, torch.fft -> cuFFT; hyena.py:388-444), as the
+    oracle restates it, on the same device, same weights, same inputs, fp32 with TF32 off: the >=10x denominator of
+    north_star."""
     import gc
-    dev = u.device
-    sd = {k: v.detach() for k, v in op.state_dict().items()}
+    from oracle import hyena_oracle as O
     B, L, D = u.shape
-    which = None
-    ref_dir = "/root/reference"
-    mod = None
-    if os.path.isdir(ref_dir):
-        try:
-            sys.path.insert(0, ref_dir)
-            import standalone_hyenadna as S
-            mod = S.HyenaOperator(D, L, order=2, filter_order=64, emb_dim=EMB, w=W_FREQ, lr_pos_emb=0.0,
-                                  modulate=True, shift=0.0).to(dev)
-            mod.load_state_dict(sd, strict=True)
-            which = "unmodified /root/reference/standalone_hyenadna.HyenaOperator on cuda"
-        except Exception as e:      # pragma: no cover
-            mod, which = None, None
-            sys.stderr.write(f"gpu_reference: reference import failed ({e!r}); using the oracle on cuda\n")
-    if mod is None:
-        from oracle import hyena_oracle as O
-        P = O.canonical(sd)
-        which = "oracle restatement (oracle/hyena_oracle.py) of the reference torch.fft path on cuda (cuFFT)"
+    P = O.canonical({k: v.detach() for k, v in op.state_dict().items()})
+    which = "oracle restatement (oracle/hyena_oracle.py) of the reference torch.fft path on cuda (cuFFT)"
 
     def one():
-        if mod is not None:
-            uu = u.detach().clone().requires_grad_(True)
-            for p in mod.parameters():
-                p.grad = None
-            mod(uu).backward(dy)
-        else:
-            O.operator_fwd_bwd(u.detach(), P, dy)
+        O.operator_fwd_bwd(u.detach(), P, dy)
 
     try:
         for _ in range(warmup):
@@ -332,7 +335,7 @@ def gpu_reference_run(op, u, dy, steps=3, warmup=1):
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1) / steps
     finally:
-        mod = None
+        P = None
         gc.collect()
         torch.cuda.empty_cache()
     return {"ms_per_step": round(ms, 3), "value": B * L / (ms * 1e-3), "unit": "nt/s", "steps": steps,
@@ -452,8 +455,9 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t_begin = sampler.mark()
     e0.record()
-    for _ in range(args.steps):
+    for _ in range(args.steps - 1):
         step()
+    y = step()
     e1.record()
     torch.cuda.synchronize()
     t_end = sampler.mark()
@@ -462,6 +466,10 @@ def main():
     prof = H._lib.profile_end()
     launches = H.launch_count() - n0
     clocks = sampler.stop(t_begin, t_end) if rank == 0 else None
+    if args.dump_outputs and rank == 0:     # before the legs below overwrite the grads
+        dump_outputs(args.dump_outputs, {"y": y, "du": u.grad,
+                                         **{"grad." + n: p.grad for n, p in op.named_parameters() if p.grad is not None}})
+    del y
     t = torch.tensor([ms], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -33,6 +33,7 @@ CASES = {
     # (modulation_lr != 0, hyena.py:145-150), with a non-zero shift
     "ref_norm_modlr_L256_D16": (2, 256, 16, 5, 10.0, 256, 0.02, 2, {"normalized": True, "modulation_lr": 1e-3, "shift": 0.05}),
 }
+TINY_SAMPLE = 8192      # stored entries of tiny_1k's y and du (of 2 * 1024 * 128 each)
 
 
 def _shim():
@@ -122,10 +123,14 @@ def main():
         for k, p in op64.named_parameters():
             out["grad64/" + k] = p.grad.numpy()
         if case == "tiny_1k":
-            # keep the fixture small: u / dy are regenerated from their seeds by the tests
-            # (checked against the checksums stored here); fp64 truth kept for the filter grads only
+            # keep the fixture small (under 1 MB): u / dy are regenerated from their seeds by the tests
+            # (checked against the checksums stored here); y / du are kept at a fixed seeded sample of
+            # TINY_SAMPLE flat indices (sample_idx); fp64 truth kept for the filter grads only
             out["u_sum"] = np.float64(u.double().sum()); out["dy_sum"] = np.float64(dy.double().sum())
             out["u_head"] = u[0, :4, :4].numpy(); out["dy_head"] = dy[0, :4, :4].numpy()
+            idx = np.sort(np.random.default_rng(0).choice(out["y"].size, TINY_SAMPLE, replace=False)).astype(np.int32)
+            out["sample_idx"] = idx
+            out["y"], out["du"] = out["y"].reshape(-1)[idx], out["du"].reshape(-1)[idx]
             for k in ("u", "dy", "y64", "du64"):
                 del out[k]
             for k in list(out):

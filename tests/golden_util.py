@@ -32,4 +32,12 @@ def load(case):
     for k in ("y", "du", "y64", "du64"):
         if k in z.files:
             out[k] = torch.from_numpy(z[k])
+    if "sample_idx" in z.files:     # outputs stored at a fixed sample of their flat indices only
+        out["sample_idx"] = torch.from_numpy(z["sample_idx"].astype(np.int64))
     return out
+
+
+def stored(G, t):
+    """The entries of an output tensor (y, du) that fixture G stores: all of them, or its fixed sample."""
+    idx = G.get("sample_idx")
+    return t if idx is None else t.reshape(-1)[idx.to(t.device)]

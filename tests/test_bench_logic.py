@@ -35,6 +35,31 @@ def test_roofline_handles_unknown_and_empty_profiles():
     assert "achieved_gbs" not in r["kernels"]["twiddle_init"]
 
 
+def test_dump_outputs_writes_whole_or_seeded_samples_within_budget(tmp_path):
+    import numpy as np
+    import torch
+    b = _bench()
+    b.DUMP_BYTES = 3 * 4 * 1000                     # 1000 float32 elements per output
+    g = torch.Generator().manual_seed(0)
+    outs = {"y": torch.randn(2, 50, 40, generator=g), "du": torch.randn(2, 50, 40, generator=g),
+            "grad.w": torch.randn(30, 20, generator=g)}
+    for d in ("a", "b"):
+        b.dump_outputs(str(tmp_path / d), outs)
+    total = 0
+    for name, t in outs.items():
+        a = np.load(tmp_path / "a" / (name + ".npy"))
+        assert a.dtype == np.float32 and np.array_equal(a, np.load(tmp_path / "b" / (name + ".npy")))
+        total += a.nbytes
+        if name == "grad.w":
+            assert np.array_equal(a, t.numpy())                     # fits its share: written whole
+        else:
+            assert a.ndim == 1 and 800 < a.size <= 1000                # 1000 draws of 4000 indices, duplicates dropped
+            assert np.isin(a, t.numpy().reshape(-1)).all()          # entries of the output, not something else
+    assert total <= b.DUMP_BYTES
+    assert np.array_equal(np.isin(outs["y"].numpy().reshape(-1), np.load(tmp_path / "a" / "y.npy")),
+                          np.isin(outs["du"].numpy().reshape(-1), np.load(tmp_path / "a" / "du.npy")))   # same indices
+
+
 def test_synthetic_inputs_match_the_oracle_recipe():
     import torch
     from oracle import hyena_oracle as O
