@@ -35,8 +35,6 @@ SIGNATURES = {
     "hyena_b200_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "hyena_b200_workspace_min_bytes": (_sz, [_i, _i, _i, _i]),
     "hyena_b200_filter_fwd": (_i, [c_fp, _i, c_fp] + [c_fp] * 7 + [c_fp, c_fp, _f, _i, _i, _i, _i, _i, c_fp, _vp]),
-    "hyena_b200_filter_bwd": (_i, [c_fp, _i, c_fp] + [c_fp] * 7 + [c_fp, c_fp, _f, _i, _i, _i, _i, _i, c_fp]
-                              + [c_fp] * 8 + [c_fp, _i, _vp]),
     "hyena_b200_filter_bwd_stage1": (_i, [c_fp, _i, c_fp] + [c_fp] * 7 + [c_fp, c_fp, _f, _i, _i, _i, _i, _i, c_fp, c_fp, c_fp, _vp]),
     "hyena_b200_filter_bwd_stage2": (_i, [c_fp] * 11 + [_i, _i, _i, _vp]),
     "hyena_b200_filter_spectrum": (_i, [c_fp, c_fp, _i, _i, _vp, _sz, _vp]),
@@ -91,7 +89,7 @@ def lib():
                 for name, (res, args) in SIGNATURES.items():
                     fn = getattr(L, name)
                     fn.restype, fn.argtypes = res, args
-                if L.hyena_b200_abi_version() != 1:
+                if L.hyena_b200_abi_version() != 2:
                     raise HyenaB200Error("libhyena_b200.so ABI version mismatch")
                 _lib = L
     return _lib

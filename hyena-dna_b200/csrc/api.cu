@@ -25,8 +25,6 @@ static bool g_prof_on = false;
 static std::vector<ProfRec> g_prof;            // records of the current profiling window
 static std::vector<cudaEvent_t> g_ev_pool;     // recycled events
 static thread_local cudaEvent_t g_cur_e0 = nullptr;
-static thread_local bool g_prof_suppress = false;   // inside a pipelined call: the kernels of different row groups overlap, so
-                                                    // the call is timed as ONE record on the caller's stream instead
 
 static cudaEvent_t get_event() {
   if (!g_ev_pool.empty()) { cudaEvent_t e = g_ev_pool.back(); g_ev_pool.pop_back(); return e; }
@@ -36,14 +34,14 @@ static cudaEvent_t get_event() {
 }
 void prof_begin(int kind, cudaStream_t s) {
   (void)kind;
-  if (!g_prof_on || g_prof_suppress) return;
+  if (!g_prof_on) return;
   std::lock_guard<std::mutex> lk(g_prof_mu);
   g_cur_e0 = get_event();
   cudaEventRecord(g_cur_e0, s);
 }
 void prof_end(int kind, cudaStream_t s) {
   g_launches.fetch_add(1, std::memory_order_relaxed);
-  if (!g_prof_on || !g_cur_e0 || g_prof_suppress) return;
+  if (!g_prof_on || !g_cur_e0) return;
   std::lock_guard<std::mutex> lk(g_prof_mu);
   cudaEvent_t e1 = get_event();
   cudaEventRecord(e1, s);
@@ -156,72 +154,6 @@ static int carve(void* ws, size_t ws_bytes, int B, int D, int L, bool backward, 
   return 0;
 }
 
-// ---------------------------------------------------------------- pipelined row groups (L2-resident scratch)
-// The three passes of a row group are enqueued back to back on one of S auxiliary streams, group g on stream g % S with
-// scratch slot g % S, G channels per group: the inter-pass scratch of a group (G x B x 8 MB at M = 2^20) is re-read while
-// it is still in the 126 MB L2, a slot is overwritten in place by the next group of its stream (dirty lines never
-// have to reach DRAM), and kernels of different groups overlap so that the short launches leave no idle tails.
-// In-stream order carries every dependency (passes of a group, reuse of a slot); the caller's stream forks into the
-// auxiliary streams and joins them again, so to the caller the call is ordered on its own stream as before.
-// HYENA_B200_PIPE="S,G" (0 = off: one launch per pass over all rows).
-struct PipeCfg { int S, G; };
-static PipeCfg pipe_cfg() {
-  static PipeCfg c = [] {
-    PipeCfg v{0, 0};
-    const char* e = getenv("HYENA_B200_PIPE");
-    int s = 0, g = 0;
-    if (e && sscanf(e, "%d,%d", &s, &g) == 2 && s >= 1 && s <= 8 && g >= 1) { v.S = s; v.G = g; }
-    return v;
-  }();
-  return c;
-}
-struct PipeDev { cudaStream_t st[8]; cudaEvent_t fork; cudaEvent_t join[8]; int n = 0; std::mutex mu; };
-static PipeDev g_pipe[64];
-static int get_pipe(int S, PipeDev** out) {
-  int dev = -1;
-  HY_CUDA(cudaGetDevice(&dev));
-  HY_CHECK(dev >= 0 && dev < 64, "unsupported device ordinal %d", dev);
-  std::lock_guard<std::mutex> lk(g_mu);
-  PipeDev& p = g_pipe[dev];
-  if (p.n == 0) HY_CUDA(cudaEventCreateWithFlags(&p.fork, cudaEventDisableTiming));
-  while (p.n < S) {
-    HY_CUDA(cudaStreamCreateWithFlags(&p.st[p.n], cudaStreamNonBlocking));
-    HY_CUDA(cudaEventCreateWithFlags(&p.join[p.n], cudaEventDisableTiming));
-    ++p.n;
-  }
-  *out = &p;
-  return 0;
-}
-// RAII: fork the caller's stream into S auxiliary streams; join() makes the caller's stream wait for all of them
-struct PipeRun {
-  PipeDev* p = nullptr; int S = 0; cudaStream_t main = nullptr; int kind = -1; bool active = false;
-  std::unique_lock<std::mutex> lk;
-  int begin(int S_, cudaStream_t main_, int kind_) {
-    S = S_; main = main_; kind = kind_;
-    if (get_pipe(S, &p)) return 1;
-    lk = std::unique_lock<std::mutex>(p->mu);
-    prof_begin(kind, main);
-    g_prof_suppress = true;
-    HY_CUDA(cudaEventRecord(p->fork, main));
-    for (int i = 0; i < S; ++i) HY_CUDA(cudaStreamWaitEvent(p->st[i], p->fork, 0));
-    active = true;
-    return 0;
-  }
-  cudaStream_t stream(int g) const { return p->st[g % S]; }
-  int join() {
-    for (int i = 0; i < S; ++i) {
-      HY_CUDA(cudaEventRecord(p->join[i], p->st[i]));
-      HY_CUDA(cudaStreamWaitEvent(main, p->join[i], 0));
-    }
-    g_prof_suppress = false;
-    active = false;
-    prof_end(kind, main);
-    g_launches.fetch_sub(1, std::memory_order_relaxed);     // the span record is not a kernel launch
-    return 0;
-  }
-  ~PipeRun() { if (active) { g_prof_suppress = false; for (int i = 0; i < S; ++i) { cudaEventRecord(p->join[i], p->st[i]); cudaStreamWaitEvent(main, p->join[i], 0); } } }
-};
-
 static int check_shape(int B, int D, int L) {
   HY_CHECK(B >= 1 && D >= 1 && L >= 1, "bad shape B=%d D=%d L=%d", B, D, L);
   HY_CHECK(L <= (1 << 20), "sequence length %d exceeds the supported maximum %d", L, 1 << 20);
@@ -275,13 +207,13 @@ HY_API int hyena_b200_profile_end(double* ms_by_kind, unsigned long long* launch
 }
 
 HY_API const char* hyena_b200_kind_name(int kind) {
-  static const char* names[K_COUNT] = {
+  static const char* names[] = {
       "col_fwd<filter>", "col_fwd<gate>", "col_fwd<dc>", "col_fwd<plain>",
       "col_inv<conv_fwd>", "col_inv<bwd_dg>", "col_inv<dk>", "col_inv<plain_fwd>", "col_inv<plain_bwd>",
       "row_pass<filter>", "row_pass<conv_fwd>", "row_pass<conv_bwd>",
-      "filter_fwd", "filter_bwd", "short_conv_bwd", "twiddle_init", "filter_tc_prep", "filter_tc_fwd", "filter_tc_bwd", "filter_tc_red", "fused_conv_fwd",
-      "spectrum_convert", "proj_prep", "proj_gemm", "proj_wgrad",
-      "conv_fwd<pipelined>", "conv_bwd<pipelined>", "filter_spectrum<pipelined>", "add_layer_norm", "filter_extra"};
+      "short_conv_bwd", "twiddle_init", "filter_tc_prep", "filter_tc_fwd", "filter_tc_bwd", "filter_tc_red",
+      "spectrum_convert", "proj_prep", "proj_gemm", "proj_wgrad", "add_layer_norm", "filter_extra"};
+  static_assert(sizeof(names) / sizeof(names[0]) == K_COUNT, "one name per Kind");
   return (kind >= 0 && kind < K_COUNT) ? names[kind] : "?";
 }
 
@@ -297,11 +229,6 @@ HY_API size_t hyena_b200_workspace_min_bytes(int B, int D, int L, int backward) 
 
 HY_API size_t hyena_b200_workspace_bytes(int B, int D, int L, int backward) {
   if (B < 1 || L < 1 || D < 1) return 0;
-  const PipeCfg pc = pipe_cfg();
-  if (pc.S > 0) {                                   // S scratch slots of G channels each
-    const int g = pc.G < D ? pc.G : D;
-    return hyena_b200_workspace_min_bytes(B, D, L, backward) * (size_t)g * (size_t)pc.S;
-  }
   int nch = channels_per_group(group_budget_bytes(), B, D, L);
   if (nch < 1) nch = 1;
   return hyena_b200_workspace_min_bytes(B, D, L, backward) * (size_t)nch;
@@ -351,28 +278,9 @@ HY_API int hyena_b200_filter_fwd(const float* z, int z_stride, const float* t, c
   if (fill_filter_params(&P, z, z_stride, t, W0, b0, W1, b1, W2, b2, W3, freq, deltas, shift, modulate, L, E, N, D))
     return 1;
   HY_CHECK(k_out, "null output");
-  static const bool simt = getenv("HYENA_B200_FILTER") && !strcmp(getenv("HYENA_B200_FILTER"), "simt");
-  if (simt) {
-    HY_CUDA(launch_filter_fwd(P, k_out, (cudaStream_t)stream));
-    return 0;
-  }
   float* wimg = nullptr;
   if (get_wimg(D, (cudaStream_t)stream, &wimg)) return 1;
   HY_CUDA(launch_filter_fwd_tc(P, wimg, k_out, (cudaStream_t)stream));
-  return 0;
-}
-
-HY_API int hyena_b200_filter_bwd(const float* z, int z_stride, const float* t, const float* W0, const float* b0,
-                          const float* W1, const float* b1, const float* W2, const float* b2, const float* W3,
-                          const float* freq, const float* deltas, float shift, int modulate, int L, int E, int N,
-                          int D, const float* dk, float* dW0, float* db0, float* dW1, float* db1, float* dW2,
-                          float* db2, float* dW3, float* dfreq, float* dz, int dz_stride, void* stream) {
-  FilterParams P;
-  if (fill_filter_params(&P, z, z_stride, t, W0, b0, W1, b1, W2, b2, W3, freq, deltas, shift, modulate, L, E, N, D))
-    return 1;
-  HY_CHECK(dk && dW0 && db0 && dW1 && db1 && dW2 && db2 && dW3 && dfreq, "null gradient pointer");
-  FilterGrads G{dW0, db0, dW1, db1, dW2, db2, dW3, dfreq, dz, dz_stride};
-  HY_CUDA(launch_filter_bwd(P, dk, G, (cudaStream_t)stream));
   return 0;
 }
 
@@ -414,21 +322,6 @@ HY_API int hyena_b200_filter_spectrum(const float* k, float* kspec, int D, int L
   PassArgs a = base_args(1, D, L, T);
   a.A = c.A; a.src = k; a.kspec_out = reinterpret_cast<float2*>(kspec);
   a.vec = ((L & 1) == 0) && aligned8(k);
-  const PipeCfg pc = pipe_cfg();
-  const int G = pc.G < D ? pc.G : D;
-  if (pc.S > 0 && c.nch >= G * pc.S && D > G) {
-    PipeRun run;
-    if (run.begin(pc.S, s, K_PIPE_FILTER)) return 1;
-    const size_t slot = (row_bytes(L) / sizeof(float2)) * (size_t)G;
-    int g = 0;
-    for (int c0 = 0; c0 < D; c0 += G, ++g) {
-      const int n = (D - c0 < G) ? D - c0 : G;
-      a.c0 = c0; a.A = c.A + slot * (size_t)(g % pc.S);
-      HY_CUDA(launch_col_fwd(COL_FILTER, a, n, run.stream(g)));
-      HY_CUDA(launch_row_pass(ROW_FILTER, a, n, run.stream(g)));
-    }
-    return run.join();
-  }
   for (int c0 = 0; c0 < D; c0 += c.nch) {
     const int n = (D - c0 < c.nch) ? D - c0 : c.nch;
     a.c0 = c0;
@@ -498,24 +391,7 @@ HY_API int hyena_b200_core_fwd(const float* p, const float* in_bias, const float
   a.p = p; a.in_bias = in_bias; a.sw = sw; a.sb = sb; a.fbias = fbias; a.out = y_pre; a.out2 = c_save;
   a.gspec = reinterpret_cast<float2*>(gspec_save);
   a.vec = ((L & 1) == 0) && aligned8(p) && aligned8(y_pre) && (!c_save || aligned8(c_save));
-  a.stage = ((L & 3) == 0) && aligned16(p) && !getenv("HYENA_B200_NO_STAGE");
-  const PipeCfg pc = pipe_cfg();
-  const int G = pc.G < D ? pc.G : D;
-  if (pc.S > 0 && c.nch >= G * pc.S && D > G) {
-    PipeRun run;
-    if (run.begin(pc.S, s, K_PIPE_FWD)) return 1;
-    const size_t slot = (row_bytes(L) / sizeof(float2)) * (size_t)B * (size_t)G;
-    int g = 0;
-    for (int c0 = 0; c0 < D; c0 += G, ++g) {
-      const int n = (D - c0 < G) ? D - c0 : G;
-      cudaStream_t st = run.stream(g);
-      a.c0 = c0; a.A = c.A + slot * (size_t)(g % pc.S);
-      HY_CUDA(launch_col_fwd(COL_GATE, a, n * B, st));
-      HY_CUDA(launch_row_pass(ROW_CONV_FWD, a, n * B, st));
-      HY_CUDA(launch_col_inv(INV_CONV_FWD, a, n * B, st));
-    }
-    return run.join();
-  }
+  a.stage = ((L & 3) == 0) && aligned16(p);
   for (int c0 = 0; c0 < D; c0 += c.nch) {
     const int n = (D - c0 < c.nch) ? D - c0 : c.nch;
     a.c0 = c0;
@@ -543,23 +419,9 @@ HY_API int hyena_b200_core_bwd(const float* dy_pre, const float* p, const float*
   a.p = p; a.in_bias = in_bias; a.sw = sw; a.sb = sb; a.fbias = fbias;
   a.vec = ((L & 1) == 0) && aligned8(p) && aligned8(dy_pre) && aligned8(c_saved) && aligned8(dk) &&
           aligned8(ds_scratch);
-  a.stage = ((L & 3) == 0) && aligned16(p) && aligned16(dy_pre) && aligned16(c_saved) && !getenv("HYENA_B200_NO_STAGE");
-  const PipeCfg pc = pipe_cfg();
-  const int G = pc.G < D ? pc.G : D;
-  const bool piped = pc.S > 0 && c.nch >= G * pc.S && D > G;
-  PipeRun run;
-  if (piped && run.begin(pc.S, s, K_PIPE_BWD)) return 1;
-  const int step = piped ? G : c.nch;
-  const size_t rowE = row_bytes(L) / sizeof(float2);
-  int g = 0;
-  for (int c0 = 0; c0 < D; c0 += step, ++g) {
-    const int n = (D - c0 < step) ? D - c0 : step;
-    if (piped) {                                  // slot g % S: [A: G*B rows][A2: G*B rows][A3: G rows]
-      s = run.stream(g);
-      c.A = reinterpret_cast<float2*>(workspace) + rowE * (size_t)(2 * B + 1) * (size_t)G * (size_t)(g % pc.S);
-      c.A2 = c.A + rowE * (size_t)B * (size_t)G;
-      c.A3 = c.A2 + rowE * (size_t)B * (size_t)G;
-    }
+  a.stage = ((L & 3) == 0) && aligned16(p) && aligned16(dy_pre) && aligned16(c_saved);
+  for (int c0 = 0; c0 < D; c0 += c.nch) {
+    const int n = (D - c0 < c.nch) ? D - c0 : c.nch;
     a.c0 = c0; a.B = B;
     a.A2 = c.A2; a.A3 = c.A3;
     a.A = c.A; a.src = dy_pre;
@@ -570,15 +432,12 @@ HY_API int hyena_b200_core_bwd(const float* dy_pre, const float* p, const float*
       HY_CUDA(launch_col_fwd(COL_GATE, a, n * B, s));    // A2 <- columns of g = v * x1 (recomputed)
     }
     a.A = c.A;
-    static const bool bwd1 = !(getenv("HYENA_B200_ROW_BWD1") && !strcmp(getenv("HYENA_B200_ROW_BWD1"), "0"));
-    // (the 128-thread batch-1 kernel exists for 1024-point rows only)
-    HY_CUDA(launch_row_pass((B == 1 && gspec_saved && bwd1 && a.logM2 == 10) ? ROW_CONV_BWD1 : ROW_CONV_BWD, a, n, s));   // A <- rows of dg, A3 <- rows of dk
+    HY_CUDA(launch_row_pass(ROW_CONV_BWD, a, n, s));     // A <- rows of dg, A3 <- rows of dk
     a.src = dy_pre; a.src2 = c_saved; a.out2 = ds_scratch; a.red = dfbias; a.dsw = dsw; a.dsb = dsb;
     HY_CUDA(launch_col_inv(INV_BWD_DG, a, n * B, s));
     a.B = 1; a.out = dk;
     HY_CUDA(launch_col_inv(INV_DK, a, n, s));
   }
-  if (piped) { if (run.join()) return 1; s = (cudaStream_t)stream; }
   // pass 3 already accumulated dsw / dsb from the operand windows it had staged: no second read of p here.
   // dp == NULL: the caller consumes ds directly (hyena_b200_proj_gemm / proj_wgrad apply the transposed short filter on
   // the fly and d in_proj.bias follows from dsb and two edge samples), so dp never exists in HBM.

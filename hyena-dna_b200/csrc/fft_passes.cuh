@@ -131,7 +131,7 @@ __device__ __forceinline__ float2 staged_pair(const float* st, int rr, int col) 
 // ------------------------------------------------------------------------------------------------
 enum ColMode { COL_FILTER = 0, COL_GATE = 1, COL_DC = 2, COL_PLAIN = 3 };
 enum InvMode { INV_CONV_FWD = 0, INV_BWD_DG = 1, INV_DK = 2, INV_PLAIN_FWD = 3, INV_PLAIN_BWD = 4 };
-enum RowMode { ROW_FILTER = 0, ROW_CONV_FWD = 1, ROW_CONV_BWD = 2, ROW_CONV_BWD1 = 3 };
+enum RowMode { ROW_FILTER = 0, ROW_CONV_FWD = 1, ROW_CONV_BWD = 2 };
 
 // Rows of one launch are numbered r = ci*B + b (all batches of a channel adjacent), channel c = c0 + ci.
 struct PassArgs {
@@ -240,15 +240,14 @@ __device__ __forceinline__ float2 col_input(const PassArgs& a, int b, int c, int
 // body of pass 1 for the column tile `bx` of row `by` (the __global__ wrapper passes blockIdx; the fused
 // cooperative kernel loops over tiles)
 template <int LOGM1, int LOGM2, int MODE>
-__device__ __forceinline__ void col_fwd_body(const PassArgs& a, const int bx, const int by, unsigned char* smem_raw,
-                                             const int c0x = 0) {
+__device__ __forceinline__ void col_fwd_body(const PassArgs& a, const int bx, const int by, unsigned char* smem_raw) {
   using CG = ColGeo<LOGM1, LOGM2>;
   constexpr int M1 = CG::M1;
   constexpr int kM2 = CG::M2;
   float2* smem = reinterpret_cast<float2*>(smem_raw);
 
   const int r = by;
-  const int ci = r / a.B, b = r - ci * a.B, c = a.c0 + c0x + ci;
+  const int ci = r / a.B, b = r - ci * a.B, c = a.c0 + ci;
   const int colbase = bx * CG::C;
   const int L = a.L;
   const bool vec = a.vec != 0;
@@ -443,15 +442,14 @@ __device__ __forceinline__ void inv_output(const PassArgs& a, InvCtx& cx, int b,
 }
 
 template <int LOGM1, int LOGM2, int MODE>
-__device__ __forceinline__ void col_inv_body(const PassArgs& a, const int bx, const int by, unsigned char* smem_raw,
-                                             const int c0x = 0) {
+__device__ __forceinline__ void col_inv_body(const PassArgs& a, const int bx, const int by, unsigned char* smem_raw) {
   using CG = ColGeo<LOGM1, LOGM2>;
   constexpr int M1 = CG::M1;
   constexpr int kM2 = CG::M2;
   float2* smem = reinterpret_cast<float2*>(smem_raw);
 
   const int r = by;
-  const int ci = r / a.B, b = r - ci * a.B, c = a.c0 + c0x + ci;
+  const int ci = r / a.B, b = r - ci * a.B, c = a.c0 + ci;
   const int colbase = bx * CG::C;
   const int L = a.L;
   const bool vec = a.vec != 0;
@@ -736,15 +734,11 @@ __device__ __forceinline__ void even_odd_filter(float2 z, float2 pc, float fb2, 
 // exchange area); CONV_BWD: rows*(EX + M2) (dc spectrum separate, g spectrum aliased onto the exchange area)
 template <int MODE, int LOGM2>
 __host__ __device__ constexpr size_t row_smem_elems(int rows) {
-  return (size_t)rows * (RowGeo<LOGM2>::EX + ((MODE == ROW_CONV_BWD || MODE == ROW_CONV_BWD1) ? RowGeo<LOGM2>::M2 : 0));
+  return (size_t)rows * (RowGeo<LOGM2>::EX + (MODE == ROW_CONV_BWD ? RowGeo<LOGM2>::M2 : 0));
 }
 
-// ROW_CONV_BWD1 is the batch-1 form of ROW_CONV_BWD with the spectrum of g saved by the forward pass: no register
-// accumulator across the batch, so it fits 128 threads x <= 170 registers and three 4-row CTAs per SM instead of one
-// 8-row CTA at 255 registers (the dc spectrum stays in shared memory between the two pointwise/inverse phases).
 template <int MODE, int LOGM2>
-__device__ __forceinline__ void row_pass_body(const PassArgs& a, const int bx, const int by, unsigned char* smem_raw,
-                                              const int c0x = 0) {
+__device__ __forceinline__ void row_pass_body(const PassArgs& a, const int bx, const int by, unsigned char* smem_raw) {
   using RG = RowGeo<LOGM2>;
   constexpr int M2 = RG::M2, TPR = RG::TPR;
   float2* smem = reinterpret_cast<float2*>(smem_raw);
@@ -762,7 +756,7 @@ __device__ __forceinline__ void row_pass_body(const PassArgs& a, const int bx, c
   float2* zbufp = smem + nslots * RG::EX + id.pslot * M2;
 
   if constexpr (MODE == ROW_FILTER) {
-    const int c = a.c0 + c0x + by;
+    const int c = a.c0 + by;
     const float2* src = a.A + (size_t)by * rowElems + (size_t)id.k1 * M2;
     float2* dst = a.kspec_out + (size_t)c * rowElems + (size_t)id.k1 * M2;
     float2 v[32];
@@ -777,18 +771,18 @@ __device__ __forceinline__ void row_pass_body(const PassArgs& a, const int bx, c
     // W_M^k for k = k1 + M1*(TPR s + q) = base * W_32^s,  base = W_M^{k1} * W_{M2}^{q}
     const float2 wbase = root20(a.T, ((uint32_t)id.k1 + ((uint32_t)q << a.logM1)) << (20 - logM));
     // skip-term coefficient of this row's channel (filter bias / D vector), doubled: see even_odd_filter
-    const int c_row = a.c0 + c0x + ((MODE == ROW_CONV_FWD) ? by / a.B : by);
+    const int c_row = a.c0 + ((MODE == ROW_CONV_FWD) ? by / a.B : by);
     const float fb2 = a.fbias ? 2.f * __ldg(a.fbias + c_row) : 0.f;
 
     if constexpr (MODE == ROW_CONV_FWD) {
       const int r = by;
-      const int ci = r / a.B, c = a.c0 + c0x + ci;
+      const int ci = r / a.B, c = a.c0 + ci;
       float2* Arow = a.A + (size_t)r * rowElems + (size_t)id.k1 * M2;
       const float2* Krow = a.kspec + (size_t)c * rowElems + (size_t)id.k1 * M2;
       const float2* Kprow = a.kspec + (size_t)c * rowElems + (size_t)id.pk1 * M2;
       row_fft_to_smem<LOGM2>(Arow, ex, ex, q, a.T, rsync);
       if (a.gspec) {                                    // keep the spectrum of g for the backward pass
-        float2* G = a.gspec + ((size_t)ci * a.B + (r - ci * a.B) + (size_t)(a.c0 + c0x) * a.B) * rowElems + (size_t)id.k1 * M2;
+        float2* G = a.gspec + ((size_t)ci * a.B + (r - ci * a.B) + (size_t)a.c0 * a.B) * rowElems + (size_t)id.k1 * M2;
         static_for<0, 32>([&](auto s_) { constexpr int s = decltype(s_)::value; G[TPR * s + q] = ex[TPR * s + q]; });
       }
       __syncthreads();
@@ -807,47 +801,8 @@ __device__ __forceinline__ void row_pass_body(const PassArgs& a, const int bx, c
       });
       __syncthreads();                                  // partner rows are done reading this row's spectrum
       row_ifft_store<LOGM2>(v, ex, Arow, q, id.k1, logM, a.T, rsync);
-    } else if constexpr (MODE == ROW_CONV_BWD1) {
-      const int ci = by, c = a.c0 + c0x + ci;            // B == 1: row index == channel index of the group
-      const float2* Krow = a.kspec + (size_t)c * rowElems + (size_t)id.k1 * M2;
-      const float2* Kprow = a.kspec + (size_t)c * rowElems + (size_t)id.pk1 * M2;
-      const float2* Grow = a.gspec + (size_t)c * rowElems + (size_t)id.k1 * M2;
-      const float2* Gprow = a.gspec + (size_t)c * rowElems + (size_t)id.pk1 * M2;
-      float2* Drow = a.A + (size_t)ci * rowElems + (size_t)id.k1 * M2;
-      row_fft_to_smem<LOGM2>(Drow, ex, zbuf, q, a.T, rsync);       // dc spectrum -> zbuf (kept for both phases)
-      __syncthreads();
-      float2 v[32];
-      static_for<0, 32>([&](auto s_) {                             // phase 1: dg spectrum = corr(dc, k)
-        constexpr int s = decltype(s_)::value;
-        const int k2 = TPR * s + q;
-        const int pc = (M2 - k2 - id.nz) & (M2 - 1);
-        float2 E, O, He, Ho;
-        even_odd(zbuf[k2], cconj(zbufp[pc]), E, O);
-        even_odd_filter(__ldg(Krow + k2), cconj(__ldg(Kprow + pc)), fb2, He, Ho);
-        const float2 WE = cmulc(E, mul_w32<s, false>(wbase));
-        float2 Ye = cadd(cmulc(E, He), cmulc(O, Ho));
-        float2 Yo = cadd(cmulc(WE, Ho), cmulc(O, He));
-        v[s] = cadd(Ye, cmul_i(Yo));
-      });
-      row_ifft_store<LOGM2>(v, ex, Drow, q, id.k1, logM, a.T, rsync);
-      rsync();
-      asm volatile("" : "+l"(Grow), "+l"(Gprow));                  // keep phase 2's loads behind phase 1 (registers)
-      static_for<0, 32>([&](auto s_) {                             // phase 2: dk spectrum = corr(dc, g)
-        constexpr int s = decltype(s_)::value;
-        const int k2 = TPR * s + q;
-        const int pc = (M2 - k2 - id.nz) & (M2 - 1);
-        float2 E, O, Ge, Go;
-        even_odd(zbuf[k2], cconj(zbufp[pc]), E, O);
-        even_odd(__ldg(Grow + k2), cconj(__ldg(Gprow + pc)), Ge, Go);
-        const float2 WE = cmulc(E, mul_w32<s, false>(wbase));
-        float2 Ke = cadd(cmulc(E, Ge), cmulc(O, Go));
-        float2 Ko = cadd(cmulc(WE, Go), cmulc(O, Ge));
-        v[s] = cadd(Ke, cmul_i(Ko));
-      });
-      float2* Krow_out = a.A3 + (size_t)ci * rowElems + (size_t)id.k1 * M2;
-      row_ifft_store<LOGM2>(v, ex, Krow_out, q, id.k1, logM, a.T, rsync);
     } else {   // ROW_CONV_BWD: loop over the batch, accumulate dK' in registers
-      const int ci = by, c = a.c0 + c0x + ci;
+      const int ci = by, c = a.c0 + ci;
       const float2* Krow = a.kspec + (size_t)c * rowElems + (size_t)id.k1 * M2;
       const float2* Kprow = a.kspec + (size_t)c * rowElems + (size_t)id.pk1 * M2;
       float2 acc[32];
@@ -859,7 +814,7 @@ __device__ __forceinline__ void row_pass_body(const PassArgs& a, const int bx, c
         row_fft_to_smem<LOGM2>(Drow, ex, zbuf, q, a.T, rsync);     // dc spectrum -> zbuf
         rsync();
         if (a.gspec) {                                             // saved by the forward pass: just load it
-          const float2* G = a.gspec + ((size_t)(a.c0 + c0x + ci) * a.B + b) * rowElems + (size_t)id.k1 * M2;
+          const float2* G = a.gspec + ((size_t)(a.c0 + ci) * a.B + b) * rowElems + (size_t)id.k1 * M2;
           static_for<0, 32>([&](auto s_) { constexpr int s = decltype(s_)::value; ex[TPR * s + q] = __ldg(G + TPR * s + q); });
         } else {
           row_fft_to_smem<LOGM2>(Grow, ex, ex, q, a.T, rsync);     // g spectrum  -> the exchange area itself
@@ -895,11 +850,13 @@ __device__ __forceinline__ void row_pass_body(const PassArgs& a, const int bx, c
   }
 }
 
-// ROW_CONV_BWD1 with the filter spectrum row and then the saved g spectrum row staged through shared memory by cp.async
-// (issued before the forward row FFT / before the first inverse FFT, so the 2 x 64 dependent __ldg's per thread of the
-// two pointwise phases -- `long_scoreboard`, the top stall of the kernel -- become shared-memory reads).  One 8 KB
-// buffer per row, reused for k then g; the partner row's buffer supplies the mirrored bins.  Shared memory per CTA:
-// rows * (EX + 2 * M2) complex = 99 KB for four rows, two CTAs per SM.  Default for batch 1 (2.75 vs 3.51 ms at large-1m, profiles/r2_ab.txt); HYENA_B200_ROW_BWD1_STAGE=0 selects the register-load form.
+// Batch-1 form of ROW_CONV_BWD with the spectrum of g saved by the forward pass: no register accumulator across the batch
+// (the dc spectrum stays in shared memory between the two pointwise/inverse phases).  The filter spectrum row and then
+// the saved g spectrum row are staged through shared memory by cp.async (issued before the forward row FFT / before the
+// first inverse FFT, so the 2 x 64 dependent __ldg's per thread of the two pointwise phases -- `long_scoreboard`, the top
+// stall of the register-load form -- become shared-memory reads).  One 8 KB buffer per row, reused for k then g; the
+// partner row's buffer supplies the mirrored bins.  Shared memory per CTA: rows * (EX + 2 * M2) complex = 99 KB for four
+// rows, two CTAs per SM.  2.75 vs 3.51 ms for the register-load form at large-1m (profiles/r2_ab.txt).
 template <int LOGM2>
 __host__ __device__ constexpr size_t row_bwd1_staged_smem_elems(int rows) {
   return (size_t)rows * (RowGeo<LOGM2>::EX + 2 * RowGeo<LOGM2>::M2);
@@ -981,9 +938,9 @@ __device__ __forceinline__ void row_bwd1_staged_body(const PassArgs& a, const in
 // ------------------------------------------------------------------------------------------------
 // Forward row pass with the filter spectrum row staged by cp.async under the forward row FFT (the register form issues 64
 // __ldg per thread right in front of the pointwise product: long_scoreboard is its top stall).  128-thread CTAs of four
-// rows, shared memory rows * (EX + M2) complex = 66.6 KB: three CTAs per SM.  Default (2.13 -> 1.98 ms at large-1m,
-// profiles/r2_ab.txt run E; a 256-thread staged form with 131 KB per CTA had lost in round 2's first sweep);
-// HYENA_B200_ROW_FWD_STAGE=0 selects the register-load form.
+// rows, shared memory rows * (EX + M2) complex = 66.6 KB: three CTAs per SM.  2.13 -> 1.98 ms at large-1m
+// (profiles/r2_ab.txt run E; a 256-thread staged form with 131 KB per CTA had lost in round 2's first sweep).  Needs a
+// 16-byte aligned kspec and M1 >= 4; otherwise row_pass_kernel<ROW_CONV_FWD> runs.
 // ------------------------------------------------------------------------------------------------
 template <int LOGM2>
 __host__ __device__ constexpr size_t row_fwd_staged_smem_elems(int rows) {
@@ -1044,7 +1001,7 @@ __device__ __forceinline__ void row_fwd_staged_body(const PassArgs& a, const int
 }
 
 template <int MODE, int LOGM2>
-__global__ void __launch_bounds__(MODE == ROW_CONV_BWD1 ? 128 : 256, MODE == ROW_CONV_BWD ? 1 : (MODE == ROW_CONV_BWD1 ? 3 : 2))
+__global__ void __launch_bounds__(256, MODE == ROW_CONV_BWD ? 1 : 2)
 row_pass_kernel(const PassArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   row_pass_body<MODE, LOGM2>(a, blockIdx.x, blockIdx.y, smem_raw);

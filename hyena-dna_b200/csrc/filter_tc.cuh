@@ -1,7 +1,7 @@
 // Implicit-filter forward on the 5th-generation tensor cores (tcgen05 / TMEM), sm_100a only.
 //
-// Same math as filter_fwd_kernel (filter_mlp.cuh; reference src/models/sequence/hyena.py:96-155,199-238),
-// but the three GEMM-shaped layers run as tcgen05.mma.kind::tf32 with fp32 accumulators in tensor memory:
+// Reference semantics in filter_params.h (src/models/sequence/hyena.py:96-155,199-238).  The three GEMM-shaped layers
+// run as tcgen05.mma.kind::tf32 with fp32 accumulators in tensor memory:
 //
 //   tile = 128 positions (UMMA M = 128, one TMEM lane per position, one thread per lane in the epilogues)
 //   layer 1,2 : D[128 x 64]  = act[128 x 64] * W^T      (N = 64,  K = 64)
@@ -18,7 +18,7 @@
 // One elected thread issues the MMAs; completion is tracked with tcgen05.commit -> mbarrier.
 #pragma once
 #include "fft_passes.cuh"
-#include "filter_mlp.cuh"
+#include "filter_params.h"
 #include "tc_prims.cuh"
 
 namespace hy {

@@ -1,6 +1,6 @@
-#define HY_FILTER_KERNEL_TU
 #include "launch.h"
 #include "filter_extra.cuh"
+#include "short_conv.cuh"
 namespace hy {
 
 // fp64 sincospi -> fp32 twiddle tables (exact argument reduction, correctly rounded to ~0.5 ulp)
@@ -19,31 +19,6 @@ cudaError_t launch_twiddle_init(float2* tw1024, float2* twlo, cudaStream_t s) {
   prof_begin(K_TWIDDLE, s);
   twiddle_init_kernel<<<4, 256, 0, s>>>(tw1024, twlo);
   prof_end(K_TWIDDLE, s);
-  return cudaGetLastError();
-}
-
-cudaError_t launch_filter_fwd(const FilterParams& P, float* kout, cudaStream_t s) {
-  const size_t smem = filter_fwd_smem(P.E);
-  cudaError_t e = set_smem(filter_fwd_kernel, smem);
-  if (e != cudaSuccess) return e;
-  prof_begin(K_FILTER_FWD, s);
-  filter_fwd_kernel<<<(P.L + kFwdTP - 1) / kFwdTP, 256, smem, s>>>(P, kout);
-  prof_end(K_FILTER_FWD, s);
-  return cudaGetLastError();
-}
-
-cudaError_t launch_filter_bwd(const FilterParams& P, const float* dk, const FilterGrads& G, cudaStream_t s) {
-  const size_t smem = filter_bwd_smem(P.E);
-  cudaError_t e = set_smem(filter_bwd_kernel, smem);
-  if (e != cudaSuccess) return e;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  const int ntiles = (P.L + kBwdTP - 1) / kBwdTP;
-  const int grid = ntiles < sms ? ntiles : sms;
-  prof_begin(K_FILTER_BWD, s);
-  filter_bwd_kernel<<<grid, 256, smem, s>>>(P, dk, G, ntiles);
-  prof_end(K_FILTER_BWD, s);
   return cudaGetLastError();
 }
 

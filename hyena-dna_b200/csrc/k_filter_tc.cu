@@ -1,6 +1,3 @@
-#include <cstdlib>
-#include <cstring>
-
 #include "launch.h"
 #include "filter_tc.cuh"
 namespace hy {
@@ -42,8 +39,7 @@ cudaError_t launch_filter_fwd_tc(const FilterParams& P, float* wimg, float* kout
   e = cudaGetLastError();
   if (e != cudaSuccess) return e;
   const int ntiles = (P.L + tc::kTileM - 1) / tc::kTileM;
-  static const bool old_form = getenv("HYENA_B200_FILTER_FWD") && !strcmp(getenv("HYENA_B200_FILTER_FWD"), "1");
-  if (P.D <= 256 && !old_form) {                    // TS form: activations in tensor memory, weights resident, two tiles in flight
+  if (P.D <= 256) {   // TS form: activations in tensor memory, weights resident, two tiles in flight
     const size_t smem = tc::fwd2_smem_bytes(P.D);
     e = set_smem(tc::filter_tc_fwd2_kernel, smem);
     if (e != cudaSuccess) return e;

@@ -1,19 +1,9 @@
 #include <cstdint>
-#include <cstdlib>
 
 #include "launch.h"
 namespace hy {
 
-// The batch-1 backward kernel at two CTAs per SM (up to 255 registers, no spills) instead of row_pass_kernel's three CTAs
-// at <= 170 registers with ~80 registers spilled: same body, 3.52 ms instead of 3.94-4.00 ms at large-1m
-// (profiles/r1_config_sweep.txt).  Default; HYENA_B200_ROW_BWD1_CTAS=3 selects the three-CTA form.
-template <int LOGM2>
-__global__ void __launch_bounds__(128, 2) row_pass_bwd1_2cta_kernel(const PassArgs a) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  row_pass_body<ROW_CONV_BWD1, LOGM2>(a, blockIdx.x, blockIdx.y, smem_raw);
-}
-
-// batch-1 backward with cp.async-staged k / g spectrum rows (fft_passes.cuh row_bwd1_staged_body): the default
+// batch-1 backward with cp.async-staged k / g spectrum rows (fft_passes.cuh row_bwd1_staged_body)
 template <int LOGM2>
 __global__ void __launch_bounds__(128, 2) row_pass_bwd1_staged_kernel(const PassArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -63,20 +53,15 @@ template <int MODE, int LOGM2>
 static cudaError_t go(const PassArgs& a, int rows, cudaStream_t s) {
   using RG = RowGeo<LOGM2>;
   const int M1 = 1 << a.logM1;
-  const int rows_cta = (MODE == ROW_CONV_BWD1) ? (RG::ROWS >= 4 ? RG::ROWS / 2 : RG::ROWS) : RG::ROWS;   // 128-thread CTAs
-  const int nslots = M1 < rows_cta ? M1 : rows_cta;
-  const int ctas = M1 < rows_cta ? 1 : M1 / rows_cta;
+  const int nslots = M1 < RG::ROWS ? M1 : RG::ROWS;
+  const int ctas = M1 < RG::ROWS ? 1 : M1 / RG::ROWS;
   const size_t smem = row_smem_elems<MODE, LOGM2>(nslots) * sizeof(float2);
   auto kern = row_pass_kernel<MODE, LOGM2>;
-  if constexpr (MODE == ROW_CONV_BWD1) {
-    static const bool three = getenv("HYENA_B200_ROW_BWD1_CTAS") && atoi(getenv("HYENA_B200_ROW_BWD1_CTAS")) == 3;
-    if (!three) kern = row_pass_bwd1_2cta_kernel<LOGM2>;
-  }
   cudaError_t e = set_smem(kern, smem);
   if (e != cudaSuccess) return e;
-  prof_begin(K_ROW + (MODE == ROW_CONV_BWD1 ? (int)ROW_CONV_BWD : MODE), s);
+  prof_begin(K_ROW + MODE, s);
   kern<<<dim3(ctas, rows), nslots * RG::TPR, smem, s>>>(a);
-  prof_end(K_ROW + (MODE == ROW_CONV_BWD1 ? (int)ROW_CONV_BWD : MODE), s);
+  prof_end(K_ROW + MODE, s);
   return cudaGetLastError();
 }
 
@@ -90,17 +75,15 @@ cudaError_t launch_row_pass(int mode, const PassArgs& a, int rows, cudaStream_t 
   switch (mode) {
     case ROW_FILTER: return by_len<ROW_FILTER>(a, rows, s);
     case ROW_CONV_FWD: {
-      static const bool staged = !(getenv("HYENA_B200_ROW_FWD_STAGE") && atoi(getenv("HYENA_B200_ROW_FWD_STAGE")) == 0);
       const bool al16 = (reinterpret_cast<uintptr_t>(a.kspec) & 15u) == 0;
-      if (staged && a.logM2 == 10 && al16 && a.logM1 >= 2) return go_fwd_staged(a, rows, s);
+      if (al16 && a.logM1 >= 2) return go_fwd_staged(a, rows, s);
       return by_len<ROW_CONV_FWD>(a, rows, s);
     }
-    case ROW_CONV_BWD: return by_len<ROW_CONV_BWD>(a, rows, s);
-    case ROW_CONV_BWD1: {
-      static const bool staged = !(getenv("HYENA_B200_ROW_BWD1_STAGE") && atoi(getenv("HYENA_B200_ROW_BWD1_STAGE")) == 0);
+    case ROW_CONV_BWD: {
+      // batch 1 with the g spectrum saved by the forward pass: the staged kernel, no accumulator across the batch
       const bool al16 = ((reinterpret_cast<uintptr_t>(a.kspec) | reinterpret_cast<uintptr_t>(a.gspec)) & 15u) == 0;
-      if (staged && a.logM2 == 10 && al16) return go_bwd1_staged(a, rows, s);
-      return by_len<ROW_CONV_BWD1>(a, rows, s);
+      if (a.B == 1 && a.gspec && al16) return go_bwd1_staged(a, rows, s);
+      return by_len<ROW_CONV_BWD>(a, rows, s);
     }
   }
   return cudaErrorInvalidValue;

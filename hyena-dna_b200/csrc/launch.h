@@ -1,8 +1,7 @@
 // Host-side launch entry points implemented in the k_*.cu translation units.
 #pragma once
 #include "fft_passes.cuh"
-#include "filter_mlp.cuh"
-#include "short_conv.cuh"
+#include "filter_params.h"
 #include "layernorm_args.h"
 
 namespace hy {
@@ -12,12 +11,11 @@ enum Kind {
   K_COL_FWD = 0,      // + ColMode  (0..3)
   K_COL_INV = 4,      // + InvMode  (4..8)
   K_ROW = 9,          // + RowMode  (9..11)
-  K_FILTER_FWD = 12, K_FILTER_BWD = 13, K_SHORT_BWD = 14, K_TWIDDLE = 15, K_FILTER_TC_PREP = 16, K_FILTER_TC_FWD = 17,
-  K_FILTER_TC_BWD = 18, K_FILTER_TC_RED = 19, K_FUSED_FWD = 20, K_CONVERT = 21, K_PROJ_PREP = 22, K_PROJ_GEMM = 23, K_PROJ_WGRAD = 24,
-  K_PIPE_FWD = 25, K_PIPE_BWD = 26, K_PIPE_FILTER = 27,   // whole pipelined calls (api.cu PipeRun): kernels of different groups overlap
-  K_ADD_LN = 28,            // residual add + LayerNorm (block glue, layernorm.cuh)
-  K_FILTER_EXTRA = 29,      // deltas gradient / channel L1 normalisation (filter_extra.cuh; non-default filter options)
-  K_COUNT = 30
+  K_SHORT_BWD = 12, K_TWIDDLE = 13, K_FILTER_TC_PREP = 14, K_FILTER_TC_FWD = 15, K_FILTER_TC_BWD = 16, K_FILTER_TC_RED = 17,
+  K_CONVERT = 18, K_PROJ_PREP = 19, K_PROJ_GEMM = 20, K_PROJ_WGRAD = 21,
+  K_ADD_LN = 22,            // residual add + LayerNorm (block glue, layernorm.cuh)
+  K_FILTER_EXTRA = 23,      // deltas gradient / channel L1 normalisation (filter_extra.cuh; non-default filter options)
+  K_COUNT = 24
 };
 void prof_begin(int kind, cudaStream_t s);     // api.cu: records an event when profiling is on
 void prof_end(int kind, cudaStream_t s);       // api.cu: records an event when profiling is on; counts the launch
@@ -26,14 +24,24 @@ cudaError_t launch_col_inv(int mode, const PassArgs& a, int rows, cudaStream_t s
 cudaError_t launch_row_pass(int mode, const PassArgs& a, int rows, cudaStream_t s);
 template <int MODE> cudaError_t launch_col_fwd_mode(const PassArgs& a, int rows, cudaStream_t s);   // k_col_fwd_m*.cu
 template <int MODE> cudaError_t launch_col_inv_mode(const PassArgs& a, int rows, cudaStream_t s);   // k_col_inv_m*.cu
-cudaError_t launch_filter_fwd(const FilterParams& P, float* kout, cudaStream_t s);
 cudaError_t launch_filter_fwd_tc(const FilterParams& P, float* wimg, float* kout, cudaStream_t s);   // k_filter_tc.cu
 size_t filter_tc_wimg_bytes(int D);
 cudaError_t launch_filter_bwd_tc(const FilterParams& P, float* wimg, const float* dk, float* dh, float* scratch, cudaStream_t s);
 struct RedLaunch { const float* dh; const float* scratch; const float* zT; float* dW0; float* db0; float* dW1; float* db1;
                    float* dW2; float* db2; float* dW3; float* dfreq; int L, D, E; };
 cudaError_t launch_filter_red_tc(const RedLaunch& r, cudaStream_t s);   // k_filter_tc.cu
-cudaError_t launch_filter_bwd(const FilterParams& P, const float* dk, const FilterGrads& G, cudaStream_t s);
+// k_filter.cu: backward of the 3-tap short filter (short_conv.cuh)
+struct ShortBwdArgs {
+  const float* ds;      // (B,3D,L)
+  const float* p;       // (B,3D,L), or null when dsw / dsb were already accumulated by pass 3
+  const float* in_bias; // (3D) or null
+  const float* sw;      // (3D,3)
+  float* dp;            // (B,3D,L)
+  float* dsw;           // (3D,3)  atomicAdd
+  float* dsb;           // (3D)    atomicAdd
+  float* dib;           // (3D)    atomicAdd (d in_proj.bias) or null
+  int L, C3, vec;
+};
 cudaError_t launch_short_bwd(const ShortBwdArgs& a, int B, cudaStream_t s);
 cudaError_t launch_twiddle_init(float2* tw1024, float2* twlo, cudaStream_t s);
 // k_proj.cu: projection GEMMs on tcgen05 (3xTF32)

@@ -6,25 +6,12 @@
 //   dp[t]  = w2 ds[t] + w1 ds[t+1] + w0 ds[t+2]          (ds[t>=L] = 0)
 //   dw_j   = sum_{b,t} ds[t] P(t-2+j),  db = sum ds,  d in_bias = sum dp
 #pragma once
-#include "fft_passes.cuh"
+#include "launch.h"
 
 namespace hy {
 
 constexpr int kScSpan = 8192;     // positions per CTA
 
-struct ShortBwdArgs {
-  const float* ds;      // (B,3D,L)
-  const float* p;       // (B,3D,L), or null when dsw / dsb were already accumulated by pass 3
-  const float* in_bias; // (3D) or null
-  const float* sw;      // (3D,3)
-  float* dp;            // (B,3D,L)
-  float* dsw;           // (3D,3)  atomicAdd
-  float* dsb;           // (3D)    atomicAdd
-  float* dib;           // (3D)    atomicAdd (d in_proj.bias) or null
-  int L, C3, vec;
-};
-
-#ifdef HY_FILTER_KERNEL_TU
 __global__ void __launch_bounds__(256) short_conv_bwd_kernel(const ShortBwdArgs a) {
   const int ch = blockIdx.y, b = blockIdx.z;
   const int L = a.L;
@@ -71,7 +58,5 @@ __global__ void __launch_bounds__(256) short_conv_bwd_kernel(const ShortBwdArgs 
     else if (a.dib) atomicAdd(a.dib + ch, s);
   }
 }
-
-#endif  // HY_FILTER_KERNEL_TU
 
 }  // namespace hy

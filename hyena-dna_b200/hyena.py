@@ -186,11 +186,8 @@ class _InProj(torch.autograd.Function):
         ctx.save_for_backward(u, W)
         B, L, D = u.shape
         C3 = W.shape[0]
-        mode = ops.proj_mode()
-        if mode == "tc":
+        if ops.proj_mode() == "tc":
             return ops.proj_gemm(u, 0, W, False, 0)                       # p (B, 3D, L) = W u^T, channel-major
-        if mode == "torch":
-            return torch.bmm(W.unsqueeze(0).expand(B, -1, -1), u.transpose(1, 2))
         p = torch.empty(B, C3, L, dtype=torch.float32, device=u.device)
         # col-major: P^T (L x 3D, ld L) = U (L x D) W^T (D x 3D);  U stored (D x L, ld D) -> op T
         ops.gemm(1, 0, L, C3, D, u, D, L * D, W, D, 0, p, L, C3 * L, batch=B)
@@ -202,32 +199,20 @@ class _InProj(torch.autograd.Function):
         B, L, D = u.shape
         C3 = W.shape[0]
         dp = dp.contiguous()
-        mode = ops.proj_mode()
-        if mode == "tc":
+        if ops.proj_mode() == "tc":
             du = ops.proj_gemm(dp, 1, W, True, 1) if ctx.needs_input_grad[0] else None      # du = dp^T W
             dW = ops.proj_wgrad(dp, u) if ctx.needs_input_grad[1] else None                 # dW = sum dp u
             return du, dW
-        if mode == "torch":
-            du = torch.matmul(dp.transpose(1, 2), W) if ctx.needs_input_grad[0] else None
-            dW = torch.bmm(dp, u).sum(0) if ctx.needs_input_grad[1] else None
-            return du, dW
         du = dW = None
-        main = torch.cuda.current_stream(u.device)
-        side = ops.side_stream(u.device) if (ctx.needs_input_grad[0] and ctx.needs_input_grad[1]) else None
         if ctx.needs_input_grad[1]:
             dW = torch.empty_like(W)
-            if side is not None:
-                side.wait_stream(main)
-            with torch.cuda.stream(side if side is not None else main):
-                # dW^T (D x 3D, ld D) = sum_b U_b^T (D x L, stored, op N) dP_b^T (L x 3D, stored ld L, op N)
-                for b in range(B):
-                    ops.gemm(0, 0, D, C3, L, u[b], D, 0, dp[b], L, 0, dW, D, 0, batch=1, beta=0.0 if b == 0 else 1.0)
+            # dW^T (D x 3D, ld D) = sum_b U_b^T (D x L, stored, op N) dP_b^T (L x 3D, stored ld L, op N)
+            for b in range(B):
+                ops.gemm(0, 0, D, C3, L, u[b], D, 0, dp[b], L, 0, dW, D, 0, batch=1, beta=0.0 if b == 0 else 1.0)
         if ctx.needs_input_grad[0]:
             du = torch.empty_like(u)
             # dU^T (D x L, ld D) = W^T (D x 3D, stored ld D, op N) dP (3D x L; stored (L x 3D, ld L) -> op T)
             ops.gemm(0, 1, D, L, C3, W, D, 0, dp, L, C3 * L, du, D, L * D, batch=B)
-        if side is not None:
-            main.wait_stream(side)
         return du, dW
 
 
@@ -241,14 +226,8 @@ class _OutProj(torch.autograd.Function):
         ctx.has_bias = b is not None
         B, C, L = y_pre.shape
         Do = W.shape[0]
-        mode = ops.proj_mode()
-        if mode == "tc":
+        if ops.proj_mode() == "tc":
             return ops.proj_gemm(y_pre, 1, W, False, 1, bias=b.contiguous() if b is not None else None)
-        if mode == "torch":
-            y = torch.bmm(y_pre.transpose(1, 2), W.t().unsqueeze(0).expand(B, -1, -1))
-            if b is not None:
-                y += b
-            return y
         y = torch.empty(B, L, Do, dtype=torch.float32, device=y_pre.device)
         # Y^T (Do x L, ld Do) = W (Do x C; stored (C x Do, ld C) -> op T) Ypre (C x L; stored (L x C, ld L) -> op T)
         ops.gemm(1, 1, Do, L, C, W, C, 0, y_pre, L, C * L, y, Do, L * Do, batch=B,
@@ -261,38 +240,23 @@ class _OutProj(torch.autograd.Function):
         B, C, L = y_pre.shape
         Do = W.shape[0]
         dy = dy.contiguous()
-        mode = ops.proj_mode()
-        if mode == "tc":
+        if ops.proj_mode() == "tc":
             d_pre = ops.proj_gemm(dy, 0, W, True, 0) if ctx.needs_input_grad[0] else None          # (B, C, L) = W^T dy^T
             dW = ops.proj_wgrad(y_pre, dy, transposed_out=True) if ctx.needs_input_grad[1] else None   # (Do, C)
             db = dy.sum((0, 1)) if (ctx.has_bias and ctx.needs_input_grad[2]) else None
             return d_pre, dW, db
-        if mode == "torch":
-            d_pre = torch.bmm(W.t().unsqueeze(0).expand(B, -1, -1), dy.transpose(1, 2)) if ctx.needs_input_grad[0] else None
-            dW = torch.bmm(dy.transpose(1, 2), y_pre.transpose(1, 2)).sum(0) if ctx.needs_input_grad[1] else None
-            db = dy.sum((0, 1)) if (ctx.has_bias and ctx.needs_input_grad[2]) else None
-            return d_pre, dW, db
         d_pre = dW = db = None
-        main = torch.cuda.current_stream(dy.device)
-        side = ops.side_stream(dy.device) if (ctx.needs_input_grad[0] and ctx.needs_input_grad[1]) else None
         if ctx.needs_input_grad[1]:
             dW = torch.empty_like(W)
-            if side is not None:
-                side.wait_stream(main)
-            with torch.cuda.stream(side if side is not None else main):
-                # dW^T (C x Do, ld C) = sum_b Ypre_b (C x L; stored (L x C, ld L) -> op T) dY_b (L x Do; stored (Do x L) -> op T)
-                for b in range(B):
-                    ops.gemm(1, 1, C, Do, L, y_pre[b], L, 0, dy[b], Do, 0, dW, C, 0, batch=1, beta=0.0 if b == 0 else 1.0)
-        # db on the caller's stream: a tensor allocated inside the side-stream context and consumed by autograd on the main
-        # stream could be handed back to side-stream work by the caching allocator while main-stream readers are pending
+            # dW^T (C x Do, ld C) = sum_b Ypre_b (C x L; stored (L x C, ld L) -> op T) dY_b (L x Do; stored (Do x L) -> op T)
+            for b in range(B):
+                ops.gemm(1, 1, C, Do, L, y_pre[b], L, 0, dy[b], Do, 0, dW, C, 0, batch=1, beta=0.0 if b == 0 else 1.0)
         if ctx.has_bias and ctx.needs_input_grad[2]:
             db = dy.sum((0, 1))
         if ctx.needs_input_grad[0]:
             d_pre = torch.empty_like(y_pre)
             # dYpre^T (L x C, ld L) = dY (L x Do; stored (Do x L, ld Do) -> op T) W (Do x C; stored (C x Do, ld C) -> op T)
             ops.gemm(1, 1, L, C, Do, dy, Do, L * Do, W, C, 0, d_pre, L, C * L, batch=B)
-        if side is not None:
-            main.wait_stream(side)
         return d_pre, dW, db
 
 
@@ -354,7 +318,7 @@ class HyenaOperator(nn.Module):
                 self._kspec_cache = (kkey, kspec)
         if self.order > 2 or self.filter_fn.bidirectional:
             y_pre = self._forward_chained(u, k, fb, l_filter)
-        elif ops.proj_mode() == "tc" and l_filter == l and ops.fuse_fir():
+        elif ops.proj_mode() == "tc" and l_filter == l:
             # one autograd node: in_proj GEMM + fused core; backward feeds ds straight into the projection GEMMs
             y_pre = ops.HyenaInCoreFn.apply(u, self.in_proj.weight, self.in_proj.bias, self.short_filter.weight,
                                             self.short_filter.bias, k, fb, kspec)

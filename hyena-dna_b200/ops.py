@@ -78,8 +78,9 @@ def filter_forward(z, t, W0, b0, W1, b1, W2, b2, W3, freq, deltas, shift, modula
     return k
 
 
-def _filter_backward_tc(z, t, W0, b0, W1, b1, W2, b2, W3, freq, deltas, shift, modulate, L, dk, need_dz):
+def filter_backward(z, t, W0, b0, W1, b1, W2, b2, W3, freq, deltas, shift, modulate, L, dk, need_dz):
     """Tensor-core backward: stage 1 on tcgen05 (csrc/filter_tc.cuh), stage 2 = sequence-length reductions."""
+    _need_cuda(z, t, W0, b0, W1, b1, W2, b2, W3, freq, deltas, dk)
     zz, tt, E, N, D = _filter_args(z, t, W0, b0, W1, b1, W2, b2, W3, freq, deltas, shift, modulate, L)
     ws = [x.contiguous() for x in (W0, b0, W1, b1, W2, b2, W3)]
     fr = freq.reshape(-1).contiguous()
@@ -105,27 +106,6 @@ def _filter_backward_tc(z, t, W0, b0, W1, b1, W2, b2, W3, freq, deltas, shift, m
         grads = [dp1 @ zz, sums[0], dp2 @ a1.t(), sums[1], dp3 @ a2.t(), sums[2], dh @ a3.t()]
         dfreq = sums[3]
     dz = (dp1.t() @ ws[0]) if need_dz else None
-    return grads, dfreq, dz
-
-
-def filter_backward(z, t, W0, b0, W1, b1, W2, b2, W3, freq, deltas, shift, modulate, L, dk, need_dz):
-    _need_cuda(z, t, W0, b0, W1, b1, W2, b2, W3, freq, deltas, dk)
-    import os
-    if os.environ.get("HYENA_B200_FILTER", "tc") != "simt":
-        return _filter_backward_tc(z, t, W0, b0, W1, b1, W2, b2, W3, freq, deltas, shift, modulate, L, dk, need_dz)
-    zz, tt, E, N, D = _filter_args(z, t, W0, b0, W1, b1, W2, b2, W3, freq, deltas, shift, modulate, L)
-    ws = [x.contiguous() for x in (W0, b0, W1, b1, W2, b2, W3)]
-    fr = freq.reshape(-1).contiguous()
-    dl = deltas.reshape(-1).contiguous()
-    dk = dk.contiguous()
-    grads = [torch.zeros_like(w) for w in ws]
-    dfreq = torch.zeros_like(fr)
-    dz = torch.zeros(L, E, dtype=torch.float32, device=z.device) if need_dz else None
-    with torch.cuda.device(z.device):
-        _lib.check(_lib.lib().hyena_b200_filter_bwd(
-            _ptr(zz), zz.stride(0), _ptr(tt), *[_ptr(w) for w in ws], _ptr(fr), _ptr(dl),
-            float(shift), int(bool(modulate)), int(L), E, N, D, _ptr(dk),
-            *[_ptr(g) for g in grads], _ptr(dfreq), _ptr(dz), E, _stream()))
     return grads, dfreq, dz
 
 
@@ -417,14 +397,12 @@ _gemm_mode = None
 
 
 def gemm_mode():
-    """'bf16x9' when the CUDA 12.9 cuBLASLt with fp32 emulation is usable, else 'torch' (torch.bmm on the
-    bundled cuBLAS).  HYENA_B200_GEMM=torch forces the latter.  Both are GPU library GEMMs."""
+    """'bf16x9' when the CUDA 12.9 cuBLASLt with fp32 emulation is usable, else 'torch' (no such library: the
+    projections then stay on the tcgen05 kernels even with the TF32 opt-in, see proj_mode)."""
     global _gemm_mode
     if _gemm_mode is None:
-        import os
-        want = os.environ.get("HYENA_B200_GEMM", "bf16x9")
         _gemm_mode = "torch"
-        if want != "torch" and torch.cuda.is_available() and _lib.lib().hyena_b200_gemm_available():
+        if torch.cuda.is_available() and _lib.lib().hyena_b200_gemm_available():
             _gemm_mode = "bf16x9"
     return _gemm_mode
 
@@ -453,24 +431,15 @@ def gemm(transa, transb, m, n, k, A, lda, strideA, B, ldb, strideB, C, ldc, stri
 
 
 _wimg_cache = {}
-_proj_mode = None
 
 
 def proj_mode():
     """'tc': the projections run on this library's tcgen05 3xTF32 kernels (csrc/proj_gemm.cuh) -- the default;
-    'lt': cuBLASLt 12.9 BF16x9 (csrc/gemm.cu; also what runs when the user opted into TF32 via
-    torch.backends.cuda.matmul.allow_tf32); 'torch': torch.bmm.  HYENA_B200_PROJ selects."""
-    global _proj_mode
-    if _proj_mode is None:
-        import os
-        want = os.environ.get("HYENA_B200_PROJ", "tc")
-        if want == "tc":
-            _proj_mode = "tc"
-        else:
-            _proj_mode = "lt" if (want != "torch" and gemm_mode() == "bf16x9") else "torch"
-    if _proj_mode == "tc" and torch.backends.cuda.matmul.allow_tf32 and gemm_mode() == "bf16x9":
-        return "lt"          # plain-TF32 opt-in: one MMA per product on the library path
-    return _proj_mode
+    'lt': cuBLASLt 12.9 in plain TF32 (csrc/gemm.cu), when the user opted into TF32 via
+    torch.backends.cuda.matmul.allow_tf32 and that library is usable: one MMA per product."""
+    if torch.backends.cuda.matmul.allow_tf32 and gemm_mode() == "bf16x9":
+        return "lt"
+    return "tc"
 
 
 def proj_gemm(act, act_layout, W, w_transposed, out_layout, bias=None, fir=None, out=None, l_range=None):
@@ -507,13 +476,6 @@ def proj_gemm(act, act_layout, W, w_transposed, out_layout, bias=None, fir=None,
 _wgrad_cache = {}
 
 
-def fuse_fir():
-    """Transposed short filter fused into the projection-backward GEMMs (default on; HYENA_B200_FUSE_FIR=0 keeps the
-    separate short_conv_bwd pass for A/B runs)."""
-    import os
-    return os.environ.get("HYENA_B200_FUSE_FIR", "1") != "0"
-
-
 def proj_wgrad(X, Y, fir=None, transposed_out=False):
     """dW (M, N) [(N, M) if transposed_out] = sum_{b,pos} X[b][m][pos] Y[b][pos][n]; X (B, M, L), Y (B, L, N)
     (csrc/proj_gemm.cuh wgrad_kernel: tcgen05 3xTF32, split-K, deterministic)."""
@@ -535,25 +497,6 @@ def proj_wgrad(X, Y, fir=None, transposed_out=False):
         _lib.check(_lib.lib().hyena_b200_proj_wgrad(_ptr(X), _ptr(Y), _ptr(fir), _ptr(dW), int(bool(transposed_out)), 0.0,
                                                     B, L, M, N, _ptr(sc), sc.numel(), _stream()))
     return dW
-
-
-_side_streams = {}
-
-
-def side_stream(device):
-    """A second stream per device for work that is independent of the main chain (weight-gradient GEMMs run there
-    while the input-gradient GEMM runs on the caller's stream: one op's cuBLASLt input scan overlaps the other's
-    tensor-core phase).  Measured on B200 at L = 2^20: no gain (39.3 vs 38.8 ms/step; both GEMMs want the whole
-    chip), so it is OFF unless HYENA_B200_SIDE_STREAM=1."""
-    import os
-    if os.environ.get("HYENA_B200_SIDE_STREAM", "0") != "1":
-        return None
-    key = device.index if device.index is not None else torch.cuda.current_device()
-    s = _side_streams.get(key)
-    if s is None:
-        s = torch.cuda.Stream(device=device)
-        _side_streams[key] = s
-    return s
 
 
 # ------------------------------------------------------------------------------------------ block glue: add + LayerNorm

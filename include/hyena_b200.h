@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define HYENA_B200_ABI_VERSION 1
+#define HYENA_B200_ABI_VERSION 2
 #if defined(__GNUC__)
 #define HY_API __attribute__((visibility("default")))
 #else
@@ -74,17 +74,8 @@ HY_API int hyena_b200_filter_fwd(const float* z, int z_stride, const float* t,
                           const float* freq, const float* deltas, float shift, int modulate,
                           int L, int E, int N, int D, float* k_out, void* stream);
 
-/* autograd of the above (the reference relies on torch autograd; closed form restated in DESIGN.md).
- * dk (D,L) -> parameter grads, all (+=) so callers zero them; dz (L,E; row stride dz_stride) may be NULL. */
-HY_API int hyena_b200_filter_bwd(const float* z, int z_stride, const float* t,
-                          const float* W0, const float* b0, const float* W1, const float* b1,
-                          const float* W2, const float* b2, const float* W3,
-                          const float* freq, const float* deltas, float shift, int modulate,
-                          int L, int E, int N, int D, const float* dk,
-                          float* dW0, float* db0, float* dW1, float* db1, float* dW2, float* db2,
-                          float* dW3, float* dfreq, float* dz, int dz_stride, void* stream);
-
-/* Tensor-core (tcgen05, 3xTF32) backward in two stages.  Stage 1: per position, recompute the activations and back-
+/* Backward of the above (the reference relies on torch autograd; closed form restated in DESIGN.md), on the tensor
+ * cores (tcgen05, 3xTF32) in two stages.  Stage 1: per position, recompute the activations and back-
  * propagate through the MLP, writing dh = dk * modulation (D,L) and seven feature-major (64,L) arrays into `scratch`
  * (7*64*L floats, 16-byte aligned): a1, a2, a3, dp1, dp2, dp3, X.  Stage 2: the parameter gradients are reductions
  * over the sequence, done as accumulating tcgen05 GEMMs with K = position (all outputs (+=); zT is z transposed,

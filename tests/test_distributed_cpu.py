@@ -100,8 +100,9 @@ def test_two_rank_gloo_allreduce_and_gather():
     assert sorted(res) == [(0, "ok"), (1, "ok")], res
 
 
-def test_c_abi_exports_every_declared_symbol():
-    """The library loads on a CPU-only box and exports exactly what include/hyena_b200.h declares."""
+def test_c_abi_v2_exports_every_declared_symbol():
+    """The library loads on a CPU-only box, reports ABI version 2 (no hyena_b200_filter_bwd) and exports exactly what
+    include/hyena_b200.h declares."""
     import re
     from importlib import import_module
     _lib = import_module("hyena_dna_b200._lib")
@@ -113,7 +114,8 @@ def test_c_abi_exports_every_declared_symbol():
     for name in declared:
         assert hasattr(L, name), f"{name} declared in include/hyena_b200.h but not exported"
     assert declared == set(_lib.SIGNATURES), (declared ^ set(_lib.SIGNATURES))
-    assert L.hyena_b200_abi_version() == 1
+    assert L.hyena_b200_abi_version() == 2
+    assert not hasattr(L, "hyena_b200_filter_bwd"), "version 2 no longer exports the CUDA-core filter backward"
     assert L.hyena_b200_max_seqlen() == 1 << 20
     assert L.hyena_b200_spectrum_elems(1000) == 1024 and L.hyena_b200_spectrum_elems(160000) == 262144
 
