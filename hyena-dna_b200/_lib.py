@@ -56,6 +56,9 @@ SIGNATURES = {
     "hyena_b200_add_layernorm_bwd": (_i, [c_fp] * 9 + [ctypes.c_longlong, _i, _vp, _sz, _vp]),
     "hyena_b200_gemm": (_i, [_i, _i, _i, _i, _i, _f, c_fp, _i, ctypes.c_longlong, c_fp, _i, ctypes.c_longlong, _f, c_fp,
                              _i, ctypes.c_longlong, _i, c_fp, _i, _vp, _sz, _vp]),
+    "hyena_b200_decode_workspace_bytes": (_sz, [_i, _i, _i]),
+    "hyena_b200_decode_prefill": (_i, [c_fp] * 6 + [_i, _i, _i, _i, _vp]),
+    "hyena_b200_decode_step": (_i, [c_fp] * 12 + [_i, _i, _i, _i, _vp, _sz, _vp]),
 }
 
 

@@ -59,9 +59,32 @@ class Block(nn.Module):
         """(hidden_states, residual) -> (mlp(LN2(.)) or mixer output, new residual); block.py:111-180, prenorm branch."""
         if mixer_subset is not None:
             raise HyenaB200Error("Block: mixer_subset is not supported")
+        return self._run(hidden_states, residual, lambda y: self.mixer(y, **(mixer_kwargs or {})))
+
+    def allocate_inference_cache(self, batch_size, max_seqlen, dtype=None, **kwargs):
+        """The mixer's decode state (HyenaOperator.allocate_inference_cache)."""
+        return self.mixer.allocate_inference_cache(batch_size, max_seqlen, dtype=dtype, **kwargs)
+
+    def prefill(self, hidden_states, residual, cache):
+        """forward() over a prompt (B, Lp, D) that also fills the mixer's decode state ``cache``."""
+        fn = self._mixer_fn("prefill")
+        return self._run(hidden_states, residual, lambda y: fn(y, cache))
+
+    def step(self, hidden_states, residual, cache):
+        """forward() for one token (B, 1, D) at the cache's position, using and advancing the mixer's decode state."""
+        fn = self._mixer_fn("step")
+        return self._run(hidden_states, residual, lambda y: fn(y, cache))
+
+    def _mixer_fn(self, name):
+        fn = getattr(self.mixer, name, None)
+        if fn is None:
+            raise HyenaB200Error(f"Block: the mixer {type(self.mixer).__name__} has no incremental decoding ({name})")
+        return fn
+
+    def _run(self, hidden_states, residual, mix):
         in_dtype = hidden_states.dtype
         y, residual = self._add_norm(hidden_states, residual, self.norm1)
-        hidden_states = self.mixer(y.to(in_dtype), **(mixer_kwargs or {}))
+        hidden_states = mix(y.to(in_dtype))
         if isinstance(hidden_states, tuple):                # mixers built with return_state
             hidden_states = hidden_states[0]
         if not isinstance(self.mlp, nn.Identity):
@@ -88,5 +111,26 @@ class Backbone(nn.Module):
         residual = None
         for layer in self.layers:
             hidden_states, residual = layer(hidden_states, residual)
+        y, _ = Block._add_norm(hidden_states, residual, self.ln_f)
+        return y.to(hidden_states.dtype)
+
+    def allocate_inference_cache(self, batch_size, max_seqlen, dtype=None, **kwargs):
+        """{layer index: decode state} for ``prefill`` / ``step``, keyed like flash_attn's InferenceParams memory dict."""
+        return {i: layer.allocate_inference_cache(batch_size, max_seqlen, dtype=dtype, **kwargs)
+                for i, layer in enumerate(self.layers)}
+
+    def prefill(self, hidden_states, caches):
+        """forward() over a prompt (B, Lp, D) that also fills every layer's decode state."""
+        residual = None
+        for i, layer in enumerate(self.layers):
+            hidden_states, residual = layer.prefill(hidden_states, residual, caches[i])
+        y, _ = Block._add_norm(hidden_states, residual, self.ln_f)
+        return y.to(hidden_states.dtype)
+
+    def step(self, hidden_states, caches):
+        """forward() for one token (B, 1, D) at the caches' position; advances every layer's decode state."""
+        residual = None
+        for i, layer in enumerate(self.layers):
+            hidden_states, residual = layer.step(hidden_states, residual, caches[i])
         y, _ = Block._add_norm(hidden_states, residual, self.ln_f)
         return y.to(hidden_states.dtype)

@@ -212,7 +212,8 @@ HY_API const char* hyena_b200_kind_name(int kind) {
       "col_inv<conv_fwd>", "col_inv<bwd_dg>", "col_inv<dk>", "col_inv<plain_fwd>", "col_inv<plain_bwd>",
       "row_pass<filter>", "row_pass<conv_fwd>", "row_pass<conv_bwd>",
       "short_conv_bwd", "twiddle_init", "filter_tc_prep", "filter_tc_fwd", "filter_tc_bwd", "filter_tc_red",
-      "spectrum_convert", "proj_prep", "proj_gemm", "proj_wgrad", "add_layer_norm", "filter_extra"};
+      "spectrum_convert", "proj_prep", "proj_gemm", "proj_wgrad", "add_layer_norm", "filter_extra",
+      "decode_prefill", "decode_step_conv", "decode_step_reduce", "decode_step_out"};
   static_assert(sizeof(names) / sizeof(names[0]) == K_COUNT, "one name per Kind");
   return (kind >= 0 && kind < K_COUNT) ? names[kind] : "?";
 }
@@ -585,6 +586,43 @@ HY_API int hyena_b200_add_layernorm_bwd(const float* dy, const float* dres, cons
   HY_CHECK(scratch_bytes >= hyena_b200_add_layernorm_scratch_bytes(rows, D), "scratch too small (%zu bytes)", scratch_bytes);
   ln::BwdArgs a{dy, dres, r, w, mean, rstd, dx, reinterpret_cast<float*>(scratch), rows, D};
   HY_CUDA(launch_add_ln_bwd(a, dw, db, (cudaStream_t)stream));
+  return 0;
+}
+
+/* incremental decoding of the order-2 operator (k_decode.cu): prompt prefill and the per-token step */
+static int check_decode_shape(int B, int D, int max_len) {
+  HY_CHECK(B >= 1 && D >= 1 && max_len >= 1, "bad decode shape B=%d D=%d max_len=%d", B, D, max_len);
+  HY_CHECK(max_len <= hyena_b200_max_seqlen(), "max_len %d exceeds the supported maximum %d", max_len,
+           hyena_b200_max_seqlen());
+  HY_CHECK(B <= decode_max_batch(), "decode batch %d exceeds the supported maximum %d", B, decode_max_batch());
+  return 0;
+}
+
+HY_API size_t hyena_b200_decode_workspace_bytes(int B, int D, int max_len) {
+  return (B < 1 || D < 1 || max_len < 1) ? 0 : decode_workspace_bytes(B, D, max_len);
+}
+
+HY_API int hyena_b200_decode_prefill(const float* p, const float* in_bias, const float* sw, const float* sb, float* g_hist,
+                                     float* fir, int B, int D, int Lp, int max_len, void* stream) {
+  if (check_decode_shape(B, D, max_len)) return 1;
+  HY_CHECK(Lp >= 1 && Lp <= max_len, "prompt length %d outside [1, max_len = %d]", Lp, max_len);
+  HY_CHECK(p && sw && sb && g_hist && fir, "null pointer");
+  HY_CUDA(launch_decode_prefill(p, in_bias, sw, sb, g_hist, fir, B, D, Lp, max_len, (cudaStream_t)stream));
+  return 0;
+}
+
+HY_API int hyena_b200_decode_step(const float* u_t, const float* W_in, const float* in_bias, const float* sw, const float* sb,
+                                  const float* k, const float* fbias, const float* W_out, const float* out_bias,
+                                  float* g_hist, float* fir, float* y_t, int B, int D, int t, int max_len,
+                                  void* workspace, size_t workspace_bytes, void* stream) {
+  if (check_decode_shape(B, D, max_len)) return 1;
+  HY_CHECK(t >= 0 && t < max_len, "position t = %d outside [0, max_len = %d)", t, max_len);
+  HY_CHECK(u_t && W_in && sw && sb && k && fbias && W_out && g_hist && fir && y_t && workspace, "null pointer");
+  HY_CHECK(workspace_bytes >= decode_workspace_bytes(B, D, max_len),
+           "decode workspace too small: %zu bytes given, %zu needed (hyena_b200_decode_workspace_bytes)", workspace_bytes,
+           decode_workspace_bytes(B, D, max_len));
+  DecodeStep d{u_t, W_in, in_bias, sw, sb, k, fbias, W_out, out_bias, g_hist, fir, y_t, B, D, t, max_len};
+  HY_CUDA(launch_decode_step(d, workspace, (cudaStream_t)stream));
   return 0;
 }
 

@@ -15,7 +15,8 @@ enum Kind {
   K_CONVERT = 18, K_PROJ_PREP = 19, K_PROJ_GEMM = 20, K_PROJ_WGRAD = 21,
   K_ADD_LN = 22,            // residual add + LayerNorm (block glue, layernorm.cuh)
   K_FILTER_EXTRA = 23,      // deltas gradient / channel L1 normalisation (filter_extra.cuh; non-default filter options)
-  K_COUNT = 24
+  K_DECODE_PREFILL = 24, K_DECODE_STEP_CONV = 25, K_DECODE_STEP_REDUCE = 26, K_DECODE_STEP_OUT = 27,   // k_decode.cu
+  K_COUNT = 28
 };
 void prof_begin(int kind, cudaStream_t s);     // api.cu: records an event when profiling is on
 void prof_end(int kind, cudaStream_t s);       // api.cu: records an event when profiling is on; counts the launch
@@ -66,6 +67,17 @@ cudaError_t launch_rfft_to_packed(const float2* X, float2* Z, int H, int logM, i
 cudaError_t launch_packed_to_rfft(const float2* Z, float2* X, int H, int logM, int logM1, float scale, cudaStream_t s);
 cudaError_t launch_rfft_to_time_small(const float2* X, float* k, int H, int L, int N, cudaStream_t s);
 cudaError_t launch_time_to_rfft_small(const float* x, float2* X, int H, int L, int N, float scale, cudaStream_t s);
+// k_decode.cu: incremental decoding (prompt prefill, per-token step)
+struct DecodeStep {
+  const float* u; const float* W_in; const float* in_bias; const float* sw; const float* sb; const float* k;
+  const float* fbias; const float* W_out; const float* out_bias; float* g_hist; float* fir; float* y;
+  int B, D, t, max_len;
+};
+size_t decode_workspace_bytes(int B, int D, int max_len);
+int decode_max_batch();
+cudaError_t launch_decode_prefill(const float* p, const float* in_bias, const float* sw, const float* sb, float* g_hist,
+                                  float* fir, int B, int D, int Lp, int max_len, cudaStream_t s);
+cudaError_t launch_decode_step(const DecodeStep& d, void* workspace, cudaStream_t s);
 
 template <class K>
 inline cudaError_t set_smem(K kernel, size_t bytes) {

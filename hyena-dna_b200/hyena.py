@@ -260,6 +260,21 @@ class _OutProj(torch.autograd.Function):
         return d_pre, dW, db
 
 
+class HyenaInferenceCache:
+    """Decode state of one HyenaOperator (see HyenaOperator.allocate_inference_cache), all fp32 on the module's device:
+    g_hist (B, D, max_seqlen) gated history, fir (B, 3D, 2) short-filter state, k (D, max_seqlen) filter, fbias (D),
+    workspace (bytes), seqlen_offset = the position the next step writes."""
+
+    def __init__(self, g_hist, fir, k, fbias, workspace):
+        self.g_hist, self.fir, self.k, self.fbias, self.workspace = g_hist, fir, k, fbias, workspace
+        self.batch_size, self.max_seqlen = g_hist.shape[0], g_hist.shape[-1]
+        self.seqlen_offset = 0
+
+    def check_batch(self, B):
+        if B != self.batch_size:
+            raise HyenaB200Error(f"batch {B} does not match the inference cache ({self.batch_size})")
+
+
 class HyenaOperator(nn.Module):
     """Hyena operator (hyena.py:270-448): order 2 as one fused pass on sm_100a, order >= 3 as a chain of its kernels.
 
@@ -332,6 +347,78 @@ class HyenaOperator(nn.Module):
         if self.return_state:
             return y, None
         return y
+
+    # ---------------------------------------------------------------------------------------- incremental decoding
+    def allocate_inference_cache(self, batch_size, max_seqlen, dtype=None, **kwargs):
+        """Decode state for ``batch_size`` sequences of up to ``max_seqlen`` positions, for ``prefill`` / ``step``.
+
+        The reference has no recurrent mode (hyena.py:384-386).  This one is exact: each step computes the causal
+        convolution over the whole stored history.  The state holds the filter k (D, max_seqlen), generated here once,
+        and the filter bias, so it is valid only while the parameters are unchanged: allocate a new one after an
+        optimizer step or a state_dict load.  The state is fp32 whatever ``dtype`` says."""
+        if self.order != 2 or self.filter_fn.bidirectional:
+            raise HyenaB200Error("incremental decoding covers the causal order-2 operator only "
+                                 f"(order={self.order}, bidirectional={self.filter_fn.bidirectional})")
+        max_seqlen, batch_size = int(max_seqlen), int(batch_size)
+        lim = min(self.l_max, 1 << 20)
+        if not 1 <= max_seqlen <= lim:
+            raise HyenaB200Error(f"max_seqlen {max_seqlen} outside [1, {lim}] (l_max = {self.l_max}, library limit 2^20)")
+        dev = self.in_proj.weight.device
+        if dev.type != "cuda":
+            raise HyenaB200Error("HyenaOperator (hyena_b200) runs on CUDA sm_100a only; there is no CPU fallback")
+        D = self.d_model
+        with torch.no_grad():
+            k = self.filter_fn.filter_channel_major(max_seqlen).detach().contiguous()
+            fb = self.filter_fn.bias if self.filter_fn.use_bias else torch.zeros_like(self.filter_fn.bias)
+            fb = fb.detach().to(torch.float32).contiguous()
+        ws = torch.empty(ops.decode_workspace_bytes(batch_size, D, max_seqlen), dtype=torch.uint8, device=dev)
+        return HyenaInferenceCache(
+            g_hist=torch.zeros(batch_size, D, max_seqlen, dtype=torch.float32, device=dev),
+            fir=torch.zeros(batch_size, 3 * D, 2, dtype=torch.float32, device=dev), k=k, fbias=fb, workspace=ws)
+
+    def prefill(self, u, cache):
+        """Run the prompt u (B, Lp, D) through the full-sequence kernels and fill ``cache`` from it.  Returns exactly what
+        ``forward(u)`` returns; the next ``step`` is position Lp.  Gradients are not tracked."""
+        B, Lp, D = u.shape
+        cache.check_batch(B)
+        if not 1 <= Lp <= cache.max_seqlen:
+            raise HyenaB200Error(f"prompt length {Lp} outside [1, max_seqlen = {cache.max_seqlen}]")
+        if not u.is_cuda:
+            raise HyenaB200Error("HyenaOperator (hyena_b200) runs on CUDA sm_100a only; there is no CPU fallback")
+        in_dtype = u.dtype
+        with torch.no_grad():
+            u = u.to(torch.float32).contiguous()
+            k = self.filter_fn.filter_channel_major(Lp)
+            fb = self.filter_fn.bias if self.filter_fn.use_bias else 0 * self.filter_fn.bias
+            W = self.in_proj.weight.contiguous()
+            # the projection and the core of forward(), run apart so that p can also feed the decode state
+            p = ops.proj_gemm(u, 0, W, False, 0) if ops.proj_mode() == "tc" else _InProj.apply(u, W)
+            y_pre = ops.HyenaCoreFn.apply(p, self.in_proj.bias, self.short_filter.weight, self.short_filter.bias, k, fb)
+            ops.decode_prefill(p, self.in_proj.bias, self.short_filter.weight.reshape(3 * D, 3), self.short_filter.bias,
+                               cache.g_hist, cache.fir)
+            y = _OutProj.apply(y_pre, self.out_proj.weight, self.out_proj.bias).to(in_dtype)
+        cache.seqlen_offset = Lp
+        return (y, None) if self.return_state else y
+
+    def step(self, u_t, cache):
+        """One token u_t (B, 1, D) at position ``cache.seqlen_offset`` -> (B, 1, D) in u_t's dtype; advances the cache.
+        Equals, to fp32 rounding, the matching row of ``forward`` over the whole sequence so far.  Gradients are not tracked."""
+        B, one, D = u_t.shape
+        cache.check_batch(B)
+        if one != 1 or D != self.d_model:
+            raise HyenaB200Error(f"step takes one token (B, 1, {self.d_model}); got {tuple(u_t.shape)}")
+        t = cache.seqlen_offset
+        if t >= cache.max_seqlen:
+            raise HyenaB200Error(f"inference cache is full: {cache.max_seqlen} positions")
+        if not u_t.is_cuda:
+            raise HyenaB200Error("HyenaOperator (hyena_b200) runs on CUDA sm_100a only; there is no CPU fallback")
+        with torch.no_grad():
+            y = ops.decode_step(u_t.reshape(B, D).to(torch.float32).contiguous(), self.in_proj.weight, self.in_proj.bias,
+                                self.short_filter.weight.reshape(3 * D, 3), self.short_filter.bias, cache.k, cache.fbias,
+                                self.out_proj.weight, self.out_proj.bias, cache.g_hist, cache.fir, t, cache.workspace)
+        cache.seqlen_offset = t + 1
+        y = y.reshape(B, 1, D).to(u_t.dtype)
+        return (y, None) if self.return_state else y
 
     def _forward_chained(self, u, k, fb, l_filter):
         """order >= 3 (the shipped HyenaDNA layer default is 3, configs/model/layer/hyena_dna.yaml:3): the recurrence of

@@ -356,6 +356,45 @@ class HyenaInCoreFn(torch.autograd.Function):
         return du, dW, dib, dsw.reshape(ctx.sw_shape), dsb, dk, dfb, None
 
 
+# ------------------------------------------------------------------------------------------ incremental decoding
+def decode_workspace_bytes(B, D, max_len):
+    return int(_lib.lib().hyena_b200_decode_workspace_bytes(int(B), int(D), int(max_len)))
+
+
+def decode_prefill(p, in_bias, sw, sb, g_hist, fir):
+    """Decode state from a prompt: g_hist[:, :, :Lp] (gated history) and fir (last two biased in_proj outputs) from the
+    prompt's p (B, 3D, Lp), the in_proj output without its bias."""
+    _need_cuda(p, in_bias, sw, sb, g_hist, fir)
+    B, C3, Lp = p.shape
+    D = C3 // 3
+    max_len = g_hist.shape[-1]
+    if not (p.is_contiguous() and g_hist.is_contiguous() and fir.is_contiguous() and C3 == 3 * D
+            and tuple(g_hist.shape) == (B, D, max_len) and tuple(fir.shape) == (B, C3, 2)):
+        raise _lib.HyenaB200Error("decode_prefill: p (B, 3D, Lp), g_hist (B, D, max_len), fir (B, 3D, 2), contiguous")
+    with torch.cuda.device(p.device):
+        _lib.check(_lib.lib().hyena_b200_decode_prefill(_ptr(p), _ptr(in_bias), _ptr(sw), _ptr(sb), _ptr(g_hist), _ptr(fir),
+                                                        B, D, Lp, max_len, _stream()))
+
+
+def decode_step(u_t, W_in, in_bias, sw, sb, k, fbias, W_out, out_bias, g_hist, fir, t, ws):
+    """One token at position t: u_t (B, D) -> y_t (B, D); appends g_t to g_hist and advances fir (csrc/k_decode.cu)."""
+    _need_cuda(u_t, W_in, in_bias, sw, sb, k, fbias, W_out, out_bias, g_hist, fir)
+    B, D = u_t.shape
+    max_len = g_hist.shape[-1]
+    for x in (u_t, W_in, in_bias, sw, sb, k, fbias, W_out, out_bias, g_hist, fir):
+        if x is not None and not x.is_contiguous():
+            raise _lib.HyenaB200Error("decode_step: every tensor must be contiguous")
+    if (tuple(W_in.shape) != (3 * D, D) or tuple(W_out.shape) != (D, D) or tuple(k.shape) != (D, max_len)
+            or tuple(g_hist.shape) != (B, D, max_len) or tuple(fir.shape) != (B, 3 * D, 2)):
+        raise _lib.HyenaB200Error("decode_step: shapes do not match u_t (B, D) and g_hist (B, D, max_len)")
+    y = torch.empty(B, D, dtype=torch.float32, device=u_t.device)
+    with torch.cuda.device(u_t.device):
+        _lib.check(_lib.lib().hyena_b200_decode_step(
+            _ptr(u_t), _ptr(W_in), _ptr(in_bias), _ptr(sw), _ptr(sb), _ptr(k), _ptr(fbias), _ptr(W_out), _ptr(out_bias),
+            _ptr(g_hist), _ptr(fir), _ptr(y), B, D, int(t), max_len, _ptr(ws), ws.numel(), _stream()))
+    return y
+
+
 # ------------------------------------------------------------------------------------------ plain fftconv
 def fftconv_forward(u, kspec, Dvec):
     _need_cuda(u, Dvec)

@@ -214,6 +214,29 @@ HY_API int hyena_b200_add_layernorm_bwd(const float* dy, const float* dres, cons
                                  const float* rstd, float* dx, float* dw, float* db, long long rows, int D, void* scratch,
                                  size_t scratch_bytes, void* stream);
 
+/* ---- incremental decoding (order 2, causal) --------------------------------------------------------
+ * The reference has no recurrent mode (hyena.py:384-386 raises NotImplementedError).  After a prompt of Lp positions has
+ * gone through the full-sequence path, every further token costs one causal dot product per channel over the history:
+ *   P[t] = W_in u_t + in_bias (3D);  s = w0 P[t-2] + w1 P[t-1] + w2 P[t] + sb (P[<0] = 0);  x0, x1, v = split(s)
+ *   g[t] = v * x1;  c[t] = sum_{j<=t} k[c][j] g[t-j] + fbias[c] g[t];  y_t = W_out (c[t] * x0) + out_bias
+ * State (owned by the caller, fp32):
+ *   g_hist (B, D, max_len)  gated history g, channel-major; positions >= the current one are never read
+ *   fir    (B, 3D, 2)       P[t-2], P[t-1] of every in_proj channel (bias included; zeros before the sequence start)
+ *   k      (D, max_len)     the filter for max_len positions (hyena_b200_filter_fwd); only k[:, :t+1] is read
+ * max_len <= hyena_b200_max_seqlen(), 1 <= B <= 64.
+ * prefill: p (B, 3D, Lp) = the prompt's in_proj output without in_proj.bias (the layout of core_fwd), 1 <= Lp <= max_len.
+ *   Writes g_hist[:, :, :Lp] and all of fir.  A fresh state starting at t = 0 needs fir zeroed and no prefill.
+ * step: position t (host int, 0 <= t < max_len), u_t (B, D) row-major, W_in (3D, D), W_out (D, D) nn.Linear layouts,
+ *   in_bias (3D) / out_bias (D) may be NULL.  Writes y_t (B, D), g_hist[:, :, t] and fir.  workspace: at least
+ *   hyena_b200_decode_workspace_bytes(B, D, max_len) bytes, 4-byte aligned.  Three kernels, deterministic (no atomics). */
+HY_API size_t hyena_b200_decode_workspace_bytes(int B, int D, int max_len);
+HY_API int hyena_b200_decode_prefill(const float* p, const float* in_bias, const float* sw, const float* sb, float* g_hist,
+                                     float* fir, int B, int D, int Lp, int max_len, void* stream);
+HY_API int hyena_b200_decode_step(const float* u_t, const float* W_in, const float* in_bias, const float* sw, const float* sb,
+                                  const float* k, const float* fbias, const float* W_out, const float* out_bias,
+                                  float* g_hist, float* fir, float* y_t, int B, int D, int t, int max_len,
+                                  void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
